@@ -59,6 +59,24 @@ def algorithmic_bytes_per_drone_step(A: int, B: int, M: int, e: int = 4, extra_o
     return e * (41 + 2 * B * A + extra_obs) + 14.0 / M
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_rows(n: int, floats_per_row: int) -> np.ndarray:
+    """Rows (envs) that --dump-outputs writes: all n if they fit DUMP_BYTES as float32 (with room for the .npy headers),
+    else a fixed seeded sample, sorted, so that every run of the same shape writes the same envs."""
+    keep = min(n, (DUMP_BYTES - 4096) // (4 * floats_per_row))
+    if keep == n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------- CPU arm
 def _cpu_worker(remote, n_envs, m, seed):
     """SubprocVecEnv worker stand-in (subproc_vec_env.py:186-261) around the oracle."""
@@ -297,10 +315,10 @@ def run_ours(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     # pre-warm (untimed, before the W warm-up steps): the process has just initialised CUDA on an idle GPU, and W = 5
     # steps are 0.2 ms of work — not enough for the SM clock to leave its idle state, and too few for the episodes to
-    # reach their stationary mix of running / re-spawning envs (nothing terminates in the first ~20 steps after a reset)
-    t_end = time.time() + args.prewarm_s
-    while time.time() < t_end:
-        gpu_steps(64, 0)
+    # reach their stationary mix of running / re-spawning envs (nothing terminates in the first ~20 steps after a reset).
+    # A step count, not a time: the timed steps then start from the same state in every run (--dump-outputs)
+    for k in range(0, args.prewarm_steps, 64):
+        gpu_steps(min(64, args.prewarm_steps - k), 0)
         torch.cuda.synchronize(dev)
     gpu_steps(args.warmup, 0)
     # (1) host in the loop: the K launches are issued while the GPU already runs the first ones.  In a 0.7 ms window
@@ -330,6 +348,13 @@ def run_ours(args):
     sync_all()
     ms = g0.elapsed_time(g1)
     launches = env.launch_count - l0
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # what the last timed step returned, gathered on the device now: the steps below overwrite the rollout slots
+        last = (args.warmup + args.steps - 1) % slots
+        rows = torch.as_tensor(dump_rows(N, M * D + 3), device=dev)
+        dump = {name: buf[last].index_select(0, rows).float() for name, buf in
+                (("obs", obs_buf), ("reward", rew_buf), ("terminated", term_buf), ("truncated", trunc_buf))}
     if ms < 300:   # keep the GPU busy a little longer so nvidia-smi sees clocks under load
         t_end = time.time() + 0.4
         while time.time() < t_end:
@@ -497,7 +522,7 @@ def run_ours(args):
                               f"({slots * N * M * D * 4 / 1e6:.0f} MB) + {slots}-slot action pool; state+history "
                               f"{(N * M * (64 + Bf * A * 4)) / 1e6:.0f} MB"),
                 "parallelism": f"env-sharded x{world}, no data-path collective",
-                "prewarm": f"{args.prewarm_s} s of untimed steps before the {args.warmup} warm-up steps (SM clock out of idle, "
+                "prewarm": f"{args.prewarm_steps} untimed steps before the {args.warmup} warm-up steps (SM clock out of idle, "
                            "episodes in their stationary running / re-spawning mix)",
                 "timed_region": "K launches of the per-step kernel between two CUDA events on the launching stream, enqueued "
                                 "behind a gate kernel the host opens when all K are queued (no host-side gaps), synchronised "
@@ -547,6 +572,8 @@ def run_ours(args):
         mappo = run_mappo_block(args, dev, rank, world)
     if line is not None and mappo is not None:
         line["mappo"] = mappo
+    if dump is not None:
+        write_outputs(args.dump_outputs, {name: t.cpu().numpy() for name, t in dump.items()})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -679,7 +706,8 @@ def main():
     ap.add_argument("--drones", type=int, default=4)
     ap.add_argument("--rollout-slots", type=int, default=16)
     ap.add_argument("--open-loop-reps", type=int, default=8, help="timed bd_step_many launches of the open-loop leg (0 = skip)")
-    ap.add_argument("--prewarm-s", type=float, default=0.3, help="seconds of untimed steps before the W warm-up steps")
+    ap.add_argument("--prewarm-steps", type=int, default=9216,
+                    help="untimed steps before the W warm-up steps (the default is about 0.3 s on one B200)")
     ap.add_argument("--e2e-steps", type=int, default=50)
     ap.add_argument("--cpu-steps", type=int, default=200)
     ap.add_argument("--vecenv-steps", type=int, default=20, help="steps of the VecEnv-protocol e2e leg (0 = skip)")
@@ -689,7 +717,15 @@ def main():
     ap.add_argument("--mappo-drones", type=int, default=16)
     ap.add_argument("--mappo-rollout", type=int, default=32)
     ap.add_argument("--mappo-minibatches", type=int, default=128)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (obs, reward, terminated, truncated of rank 0) as "
+                         "DIR/<name>.npy in float32; a fixed seeded sample of the envs when they exceed 64 MB. The inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     if args.impl == "reference":
         args.steps = 24 if args.steps is None else args.steps
         args.warmup = 3 if args.warmup is None else args.warmup

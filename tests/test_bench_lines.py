@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -68,5 +69,26 @@ def test_committed_reference_arm_line():
 def test_bench_cli_defaults():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+
+
+def test_bench_rejects_a_run_without_timed_steps():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
+def test_dumped_outputs_are_a_fixed_sample_under_64_mb(tmp_path):
+    import bench
+    N, M, D = 65536, 4, 72                                   # the default workload: obs (N, M, D), three (N,) arrays
+    rows = bench.dump_rows(N, M * D + 3)
+    assert np.array_equal(rows, bench.dump_rows(N, M * D + 3))
+    assert np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < N and len(rows) > N // 2
+    assert np.array_equal(bench.dump_rows(1000, M * D + 3), np.arange(1000))
+    n = len(rows)
+    bench.write_outputs(str(tmp_path / "out"), {"obs": np.zeros((n, M, D), np.float32), "reward": np.zeros(n, np.float32),
+                                                "terminated": np.zeros(n, np.float32), "truncated": np.zeros(n, np.float32)})
+    files = sorted(os.listdir(tmp_path / "out"))
+    assert files == ["obs.npy", "reward.npy", "terminated.npy", "truncated.npy"]
+    assert sum(os.path.getsize(tmp_path / "out" / f) for f in files) <= 64_000_000
