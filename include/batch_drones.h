@@ -225,6 +225,18 @@ int bd_set_controller_state(bd_handle* h, const void* ctrl9_dev, void* stream);
  * when the policy hands float32 actions to the reference (BaseRLAviary.py:192). */
 int bd_set_action_f32(bd_handle* h, int is_f32);
 
+/* L2 residency plan of the fast step kernel (DESIGN.md section 4).  Between two steps of a tile the
+ * state planes, step counters and episode returns (*keep_state = 1) and the keep_slots newest action-ring
+ * slots (*keep_slots, 0 .. buf_slots-1) are marked evict_last; everything read for the last time is marked
+ * evict_first.  The budget rule keeps the state first, then as many slots as fit, in what the device's L2
+ * (l2_bytes) can hold; *keep_state = 0 when the state alone does not fit.  `force` is the BD_L2_KEEP
+ * override ("off", "state", or a slot count k: the state plus k slots) or NULL.  Host computation only;
+ * BD_EINVAL for a malformed override or shape.  bd_create runs it with the device's L2 size and BD_L2_KEEP. */
+int bd_l2_plan(int n_envs, int n_drones, int act_dim, int buf_slots, int track_episodes, int64_t l2_bytes,
+               const char* force, int* keep_state, int* keep_slots);
+/* The plan a handle's step kernel runs with (both 0 when the handle does not use the fast tile kernel). */
+int bd_l2_policy(const bd_handle* h, int* keep_state, int* keep_slots);
+
 int bd_obs_dim(const bd_handle* h);              /* D                                 */
 int bd_act_dim(const bd_handle* h);              /* A                                 */
 int bd_action_buffer_size(const bd_handle* h);   /* B                                 */

@@ -22,7 +22,7 @@ BD_RESET = {"fixed": 0, "jitter_philox": 1, "jitter_buffer": 2}
 EXPORTS = (
     "bd_create", "bd_destroy", "bd_set_init_poses", "bd_set_jitter", "bd_reset", "bd_step",
     "bd_step_host", "bd_step_host_compact", "bd_step_many", "bd_set_step_many_mode", "bd_stream_gate", "bd_get_rng_state", "bd_set_rng_state",
-    "bd_debug_set_tile_epoch", "bd_get_state", "bd_set_state", "bd_get_targets", "bd_episode_stats",
+    "bd_debug_set_tile_epoch", "bd_l2_plan", "bd_l2_policy", "bd_get_state", "bd_set_state", "bd_get_targets", "bd_episode_stats",
     "bd_get_controller_state", "bd_set_controller_state", "bd_set_action_f32", "bd_obs_dim", "bd_act_dim",
     "bd_action_buffer_size", "bd_substeps", "bd_launch_count", "bd_last_error", "bd_version",
     "bd_actor_create", "bd_actor_destroy", "bd_actor_set_weights", "bd_actor_forward", "bd_actor_set_trace", "bd_actor_launch_count",
@@ -125,6 +125,11 @@ def load():
     for name in ("bd_obs_dim", "bd_act_dim", "bd_action_buffer_size", "bd_substeps"):
         getattr(lib, name).argtypes = [vp]
         getattr(lib, name).restype = C.c_int
+    ip = C.POINTER(C.c_int)
+    lib.bd_l2_plan.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_char_p, ip, ip]
+    lib.bd_l2_plan.restype = C.c_int
+    lib.bd_l2_policy.argtypes = [vp, ip, ip]
+    lib.bd_l2_policy.restype = C.c_int
     lib.bd_launch_count.argtypes = [vp]
     lib.bd_launch_count.restype = C.c_int64
     lib.bd_last_error.argtypes = []

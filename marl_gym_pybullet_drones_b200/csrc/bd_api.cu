@@ -66,6 +66,7 @@ struct bd_handle {
   int* tile_epoch = nullptr;
   unsigned long long* finished = nullptr;
   int pipeline = 0;
+  int l2_keep_state = 0, l2_keep_slots = 0;   // fast tile kernel's L2 residency plan (bd_l2_plan)
   float* ep_ret = nullptr;
   double* ep_acc = nullptr;
   void* ctrl = nullptr;        // DSL PID memory + commanded rpm, PID action types only
@@ -116,6 +117,7 @@ void fill_params(const bd_handle* h, bd::Params<R>& P) {
   P.hist = h->hist; P.stepc = h->stepc; P.gsteps = h->gsteps; P.tile_epoch = h->tile_epoch; P.finished = h->finished;
   P.step_tiles = h->spec.impl == 1 ? (h->cfg.n_envs + 4 * h->EW - 1) / (4 * h->EW) : (h->cfg.n_envs + h->E - 1) / h->E;
   P.pipeline = h->pipeline; P.pipe_wait = 0; P.early_prefetch = 0; P.ep_ret = h->ep_ret; P.ep_acc = h->ep_acc;
+  P.l2_keep_state = h->l2_keep_state; P.l2_keep_slots = h->l2_keep_slots;
   P.ctrl = (R*)h->ctrl;
   P.act_type = c.act_type; P.ctrl_reset = c.ctrl_reset_on_reset;
   P.ctrl_dt = (R)(1.0 / c.ctrl_freq);                      // CTRL_TIMESTEP (BaseAviary.py:83)
@@ -353,6 +355,11 @@ int bd_create(const bd_config* cfg, bd_handle** out) {
   if (pe != cudaSuccess) { delete h; return fail(BD_ECUDA, "cudaGetDeviceProperties: %s", cudaGetErrorString(pe)); }
   if (h->spec.impl == 1 && (size_t)(4 * h->EW) * cfg->n_drones * h->D * 4 > prop.sharedMemPerBlockOptin) h->spec.impl = 0;
   h->spec.sm_count = prop.multiProcessorCount;
+  if (h->spec.impl == 1) {
+    const int rc = bd_l2_plan(cfg->n_envs, cfg->n_drones, h->A, h->B, cfg->track_episodes, prop.l2CacheSize,
+                              getenv("BD_L2_KEEP"), &h->l2_keep_state, &h->l2_keep_slots);
+    if (rc) { delete h; return rc; }
+  }
   if (smem > prop.sharedMemPerBlockOptin) {
     delete h;
     return fail(BD_EINVAL, "bd_create: the history staging tile needs %zu B of shared memory (> %zu)", smem,
@@ -907,6 +914,47 @@ int bd_episode_stats(bd_handle* h, double* stats3_dev, int reset, void* stream) 
   cudaError_t e = bd::launch_episode_stats(h->ep_acc, stats3_dev, reset, (cudaStream_t)stream);
   h->launches++;
   if (e != cudaSuccess) return fail(BD_ECUDA, "episode_stats kernel launch failed: %s", cudaGetErrorString(e));
+  return BD_OK;
+}
+
+int bd_l2_plan(int n_envs, int n_drones, int act_dim, int buf_slots, int track_episodes, int64_t l2_bytes,
+               const char* force, int* keep_state, int* keep_slots) {
+  if (!keep_state || !keep_slots) return fail(BD_EINVAL, "bd_l2_plan: null output");
+  if (n_envs < 1 || n_drones < 1 || act_dim < 1 || buf_slots < 1 || l2_bytes < 0)
+    return fail(BD_EINVAL, "bd_l2_plan: bad shape");
+  *keep_state = 0;
+  *keep_slots = 0;
+  if (force && *force) {   // an empty override counts as unset
+    if (strcmp(force, "off") == 0) return BD_OK;
+    *keep_state = 1;
+    if (strcmp(force, "state") == 0) return BD_OK;
+    char* end = nullptr;
+    const long k = strtol(force, &end, 10);
+    if (end == force || *end != '\0' || k < 0) {
+      *keep_state = 0;
+      return fail(BD_EINVAL, "BD_L2_KEEP=%s: expected off, state or a slot count", force);
+    }
+    *keep_slots = (int)(k < buf_slots - 1 ? k : buf_slots - 1);
+    return BD_OK;
+  }
+  const long long n = (long long)n_envs * n_drones;
+  const long long state = n * 64 + (long long)n_envs * (track_episodes ? 8 : 4);   // 4 float4 planes, counter, return
+  const long long slot = n * act_dim * 4;
+  // evict_last bytes that still pay off, measured (profiles/README.md, "L2 residency budget"): 3/10 of the L2, about
+  // 40 MB on a B200.  Beyond it the step gets slower again — kept lines crowd out the streaming traffic, and every tile
+  // runs on a different SM each step, so a line may be wanted in both L2 partitions.
+  const long long budget = l2_bytes * 3 / 10;
+  if (state > budget) return BD_OK;
+  *keep_state = 1;
+  const long long k = (budget - state) / slot;
+  *keep_slots = (int)(k < buf_slots - 1 ? k : buf_slots - 1);
+  return BD_OK;
+}
+
+int bd_l2_policy(const bd_handle* h, int* keep_state, int* keep_slots) {
+  if (!h || !keep_state || !keep_slots) return fail(BD_EINVAL, "bd_l2_policy: null argument");
+  *keep_state = h->l2_keep_state;
+  *keep_slots = h->l2_keep_slots;
   return BD_OK;
 }
 

@@ -44,6 +44,17 @@ __device__ __forceinline__ void cp_async(void* smem_dst, const void* gmem_src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], %2;\n" ::"r"(d), "l"(gmem_src), "n"(BYTES) : "memory");
   }
 }
+// the same with an L2 eviction-priority descriptor (createpolicy), see L2Hints
+template <int BYTES>
+__device__ __forceinline__ void cp_async_hint(void* smem_dst, const void* gmem_src, uint64_t pol) {
+  unsigned d = static_cast<unsigned>(__cvta_generic_to_shared(smem_dst));
+  if constexpr (BYTES == 16) {
+    asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;\n" ::"r"(d), "l"(gmem_src), "l"(pol) : "memory");
+  } else {
+    asm volatile("cp.async.ca.shared.global.L2::cache_hint [%0], [%1], %2, %3;\n" ::"r"(d), "l"(gmem_src), "n"(BYTES), "l"(pol)
+                 : "memory");
+  }
+}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;\n" ::: "memory"); }
 
@@ -817,29 +828,103 @@ __device__ __forceinline__ void bulk_store_s2g(void* gdst, const void* ssrc, uin
                : "memory");
   asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
 }
+// L2 residency budget of the fast step kernel (DESIGN.md section 4): what the same tile reads again next step is
+// marked evict_last, as far as the handle's budget (Params::l2_keep_state / l2_keep_slots) allows; data read for the
+// last time is marked evict_first so that it goes before anything kept.  A ring slot's age is the number of steps
+// since it was written (0: written by this step, read again at ages 1 .. B-1).  With the policy off every access
+// carries evict_normal, the priority of an access without a hint.  Hints only choose where bytes come from.
+__device__ __forceinline__ uint64_t l2_pol_last() {
+  uint64_t p;
+  asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;\n" : "=l"(p));
+  return p;
+}
+__device__ __forceinline__ uint64_t l2_pol_first() {
+  uint64_t p;
+  asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(p));
+  return p;
+}
+__device__ __forceinline__ uint64_t l2_pol_normal() {
+  uint64_t p;
+  asm("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;\n" : "=l"(p));
+  return p;
+}
+struct L2Hints {
+  uint64_t state;       // state planes, step counter, episode return
+  uint64_t slot_keep;   // ring slots younger than keep_slots
+  uint64_t slot_drop;   // ring slots at or beyond keep_slots
+  uint64_t once;        // caller's actions: read once
+  int keep_slots;
+};
+template <typename R>
+__device__ __forceinline__ L2Hints l2_hints(const Params<R>& P) {
+  const uint64_t last = l2_pol_last(), first = l2_pol_first(), normal = l2_pol_normal();
+  const bool on = P.l2_keep_state || P.l2_keep_slots > 0;
+  return {P.l2_keep_state ? last : normal, last, on ? first : normal, first, P.l2_keep_slots};
+}
+__device__ __forceinline__ uint64_t l2_slot_pol(const L2Hints& h, int age) { return age < h.keep_slots ? h.slot_keep : h.slot_drop; }
+
+__device__ __forceinline__ float4 ld_hint(const float4* p, uint64_t pol) {
+  float4 v;
+  asm volatile("ld.global.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;\n"
+               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol) : "memory");
+  return v;
+}
+__device__ __forceinline__ float ld_hint(const float* p, uint64_t pol) {
+  float v;
+  asm volatile("ld.global.L2::cache_hint.f32 %0, [%1], %2;\n" : "=f"(v) : "l"(p), "l"(pol) : "memory");
+  return v;
+}
+__device__ __forceinline__ int ld_hint(const int* p, uint64_t pol) {
+  int v;
+  asm volatile("ld.global.L2::cache_hint.s32 %0, [%1], %2;\n" : "=r"(v) : "l"(p), "l"(pol) : "memory");
+  return v;
+}
+__device__ __forceinline__ void st_hint(float4* p, float4 v, uint64_t pol) {
+  asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;\n" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w),
+               "l"(pol)
+               : "memory");
+}
+__device__ __forceinline__ void st_hint(float* p, float v, uint64_t pol) {
+  asm volatile("st.global.L2::cache_hint.f32 [%0], %1, %2;\n" ::"l"(p), "f"(v), "l"(pol) : "memory");
+}
+__device__ __forceinline__ void st_hint(int* p, int v, uint64_t pol) {
+  asm volatile("st.global.L2::cache_hint.s32 [%0], %1, %2;\n" ::"l"(p), "r"(v), "l"(pol) : "memory");
+}
+
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all0() { asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
 
 // action history of one tile, oldest -> second newest (BaseRLAviary.py:317-318): time-ordered
-// entries j in [j0, j1) of B-1, entry j = ring slot (head+1+j) % B -> columns 12+jA.. of my row.
-template <int A, bool VEC>
-__device__ __forceinline__ void history_run(float*& dst, const float* src, size_t plane, int n) {
+// entries j in [j0, j1) of B-1, entry j = ring slot (head+1+j) % B (age B-1-j) -> columns 12+jA.. of my row.
+// HINT: each copy carries the L2 policy of its slot's age (L2Hints).
+template <int A, bool VEC, bool HINT>
+__device__ __forceinline__ void history_run(float*& dst, const float* src, size_t plane, int n, int& age, const L2Hints& h) {
 #pragma unroll 2
   for (int j = 0; j < n; ++j) {
-    if constexpr (VEC) cp_async<16>(dst, src);
-    else {
+    if constexpr (HINT) {
+      const uint64_t pol = l2_slot_pol(h, age);
+      if constexpr (VEC) cp_async_hint<16>(dst, src, pol);
+      else {
 #pragma unroll
-      for (int k = 0; k < A; ++k) cp_async<4>(dst + k, src + k);
+        for (int k = 0; k < A; ++k) cp_async_hint<4>(dst + k, src + k, pol);
+      }
+    } else {
+      if constexpr (VEC) cp_async<16>(dst, src);
+      else {
+#pragma unroll
+        for (int k = 0; k < A; ++k) cp_async<4>(dst + k, src + k);
+      }
     }
     dst += A;
     src += plane;
+    --age;
   }
 }
 
-template <typename R, int A, bool VEC>
+template <typename R, int A, bool VEC, bool HINT = false>
 __device__ __forceinline__ void issue_history(const Params<R>& P, long long g, int head, float* myrow,
-                                              int j0, int j1) {
+                                              int j0, int j1, const L2Hints& h = L2Hints{}) {
   if (g < P.n_total) {
     const size_t plane = (size_t)P.n_total * A;
     const float* base = P.hist + (size_t)g * A;
@@ -847,12 +932,13 @@ __device__ __forceinline__ void issue_history(const Params<R>& P, long long g, i
     // entries j0..j1-1 = slots head+1+j0 .. ; split at the ring wrap into two straight runs
     const int s0 = head + 1 + j0;            // may be >= B
     const int n = j1 - j0;
+    int age = P.B - 1 - j0;
     if (s0 >= P.B) {
-      history_run<A, VEC>(dst, base + (size_t)(s0 - P.B) * plane, plane, n);
+      history_run<A, VEC, HINT>(dst, base + (size_t)(s0 - P.B) * plane, plane, n, age, h);
     } else {
       const int n1 = min(n, P.B - s0);
-      history_run<A, VEC>(dst, base + (size_t)s0 * plane, plane, n1);
-      history_run<A, VEC>(dst, base, plane, n - n1);
+      history_run<A, VEC, HINT>(dst, base + (size_t)s0 * plane, plane, n1, age, h);
+      history_run<A, VEC, HINT>(dst, base, plane, n - n1, age, h);
     }
   }
 }

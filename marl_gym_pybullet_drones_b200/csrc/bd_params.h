@@ -76,6 +76,10 @@ struct Params {
   unsigned long long seed;
   int obs_aligned;                // 1: the caller's observation pointer is 16-byte aligned (bulk / 128-bit row stores allowed)
   uint32_t philox_base;           // added to the step count in the Philox counter (bd_set_rng_state: resumed runs continue the stream)
+  // fast tile kernel's L2 residency budget (bd_l2_plan, DESIGN.md section 4): state planes, step counter and episode
+  // return evict_last; ring slots younger than l2_keep_slots (0 .. B-1) evict_last, older ones evict_first
+  int l2_keep_state;
+  int l2_keep_slots;
 };
 
 struct LaunchSpec {

@@ -18,7 +18,8 @@
 // the MultiHover re-spawn rule use warp shuffles (envs are lane groups, M | 32), so there
 // is no reduction scratch; (4) one __syncthreads, then the 128 finished rows (36 864 B for
 // D = 72) leave as ONE TMA bulk store issued by thread 0; state planes and the ring slot
-// are plain 128-bit stores.
+// are 128-bit stores.  Every global access carries an L2 eviction priority (L2Hints): what
+// the tile reads again next step is kept in L2 as far as the handle's budget allows.
 // Dependency on the previous control step (0): per tile, not per grid.  A CTA waits (ld.acquire) for the
 // epoch its own tile's previous CTA published (st.release) instead of griddepcontrol.wait, so back-to-back
 // launches overlap tile by tile; a per-launch decision (bd_device.cuh: pipe_gate) falls back to the
@@ -40,13 +41,21 @@ struct TileIn {
   float ep_ret;
 };
 
-// the handle's own data (written by the previous step of this tile) ...
-template <int A>
-__device__ __forceinline__ void load_state(const Params<float>& P, long long g, int env, bool active, TileIn<A>& in) {
+// the handle's own data (written by the previous step of this tile) ...   HINT: with the L2 policies of L2Hints
+template <int A, bool HINT = false>
+__device__ __forceinline__ void load_state(const Params<float>& P, long long g, int env, bool active, TileIn<A>& in,
+                                           const L2Hints& h = L2Hints{}) {
   if (active) {
-    in.s0 = P.s0[g]; in.s1 = P.s1[g]; in.s2 = P.s2[g]; in.s3 = P.s3[g];
-    in.stepc = P.stepc[env];
-    in.ep_ret = P.ep_ret != nullptr ? P.ep_ret[env] : 0.f;
+    if constexpr (HINT) {
+      in.s0 = ld_hint(P.s0 + g, h.state); in.s1 = ld_hint(P.s1 + g, h.state);
+      in.s2 = ld_hint(P.s2 + g, h.state); in.s3 = ld_hint(P.s3 + g, h.state);
+      in.stepc = ld_hint(P.stepc + env, h.state);
+      in.ep_ret = P.ep_ret != nullptr ? ld_hint(P.ep_ret + env, h.state) : 0.f;
+    } else {
+      in.s0 = P.s0[g]; in.s1 = P.s1[g]; in.s2 = P.s2[g]; in.s3 = P.s3[g];
+      in.stepc = P.stepc[env];
+      in.ep_ret = P.ep_ret != nullptr ? P.ep_ret[env] : 0.f;
+    }
   } else {
     in.s0 = in.s1 = in.s2 = in.s3 = make_float4(0.f, 0.f, 0.f, 0.f);
     in.s1.z = 1.0f;
@@ -55,11 +64,17 @@ __device__ __forceinline__ void load_state(const Params<float>& P, long long g, 
   }
 }
 // ... and the caller's (possibly written by the kernel enqueued just before this launch)
-template <int A>
-__device__ __forceinline__ void load_action(const Params<float>& P, long long g, bool active, TileIn<A>& in) {
+template <int A, bool HINT = false>
+__device__ __forceinline__ void load_action(const Params<float>& P, long long g, bool active, TileIn<A>& in,
+                                            const L2Hints& h = L2Hints{}) {
   if (active) {
-    if constexpr (A == 4) in.act = reinterpret_cast<const float4*>(P.actions)[g];
-    else in.act = make_float4(reinterpret_cast<const float*>(P.actions)[g], 0.f, 0.f, 0.f);
+    if constexpr (HINT) {
+      if constexpr (A == 4) in.act = ld_hint(reinterpret_cast<const float4*>(P.actions) + g, h.once);
+      else in.act = make_float4(ld_hint(reinterpret_cast<const float*>(P.actions) + g, h.once), 0.f, 0.f, 0.f);
+    } else {
+      if constexpr (A == 4) in.act = reinterpret_cast<const float4*>(P.actions)[g];
+      else in.act = make_float4(reinterpret_cast<const float*>(P.actions)[g], 0.f, 0.f, 0.f);
+    }
   } else {
     in.act = make_float4(0.f, 0.f, 0.f, 0.f);
   }
@@ -167,6 +182,7 @@ step_kernel_tile(const __grid_constant__ Params<float> P) {
   float* myrow = tile_s + (size_t)(env_w < EW ? env_l * M + drone : 0) * D;   // idle lanes alias a live row, never write
   const bool jit = (TASK == TASK_MULTIHOVER) && (P.reset_mode != RESET_FIXED);
   const long long gh = active ? g : P.n_total;          // idle lanes issue no history copies
+  const L2Hints l2 = l2_hints(P);
 
   // ---- 1. every load of the tile is issued before anything is consumed ------------------------
   // Programmatic dependent launch: this grid may become resident while the previous kernel of
@@ -188,23 +204,23 @@ step_kernel_tile(const __grid_constant__ Params<float> P) {
     total = P.host_total;
     head = P.host_head;
     if (pipe_gate(P, tile, total, tid)) pdl_wait();
-    issue_history<float, A, VEC>(P, gh, head, myrow, 0, B - 2);
+    issue_history<float, A, VEC, true>(P, gh, head, myrow, 0, B - 2, l2);
   } else if (P.host_total >= 0 && P.early_prefetch) {
     total = P.host_total;
     head = P.host_head;   // = total % B (ring slot overwritten by this step's action), divided on the host
-    issue_history<float, A, VEC>(P, gh, head, myrow, 0, B - 2);
+    issue_history<float, A, VEC, true>(P, gh, head, myrow, 0, B - 2, l2);
     pdl_wait();
   } else {              // CUDA-graph mode (the step count is read from device memory), or a grid smaller than the
     pdl_wait();         // resident capacity (several earlier launches could still be in flight: no early reads)
     total = P.host_total >= 0 ? P.host_total : P.gsteps[0];   // only the last CTA to finish modifies it, after every read
     head = total % B;
-    issue_history<float, A, VEC>(P, gh, head, myrow, 0, B - 2);
+    issue_history<float, A, VEC, true>(P, gh, head, myrow, 0, B - 2, l2);
   }
   TileIn<A> cur;
-  load_state<A>(P, g, env, active, cur);
-  issue_history<float, A, VEC>(P, gh, head, myrow, B - 2, B - 1);
+  load_state<A, true>(P, g, env, active, cur, l2);
+  issue_history<float, A, VEC, true>(P, gh, head, myrow, B - 2, B - 1, l2);
   cp_async_commit();
-  load_action<A>(P, g, active, cur);
+  load_action<A, true>(P, g, active, cur, l2);
   const int stepc = cur.stepc;
   // drag reads last_clipped_action during the first substep (BaseAviary.py:359,372): the previous step's action,
   // i.e. ring slot head-1; zero right after a reset (:468)
@@ -265,10 +281,10 @@ step_kernel_tile(const __grid_constant__ Params<float> P) {
     if constexpr (A == 4) {
       if (vec) *reinterpret_cast<float4*>(myrow + 12 + (B - 1) * 4) = cur.act;
       else { float* o = myrow + 12 + (B - 1) * 4; o[0] = cur.act.x; o[1] = cur.act.y; o[2] = cur.act.z; o[3] = cur.act.w; }
-      *reinterpret_cast<float4*>(P.hist + ((size_t)head * P.n_total + g) * 4) = cur.act;
+      st_hint(reinterpret_cast<float4*>(P.hist + ((size_t)head * P.n_total + g) * 4), cur.act, l2_slot_pol(l2, 0));
     } else {
       myrow[12 + B - 1] = cur.act.x;
-      P.hist[(size_t)head * P.n_total + g] = cur.act.x;
+      st_hint(P.hist + (size_t)head * P.n_total + g, cur.act.x, l2_slot_pol(l2, 0));
     }
   }
 
@@ -306,7 +322,7 @@ step_kernel_tile(const __grid_constant__ Params<float> P) {
     P.reward[env] = reward;
     P.terminated[env] = terminated ? 1 : 0;
     P.truncated[env] = truncated ? 1 : 0;
-    P.stepc[env] = done_reset ? 0 : stepc + P.S;
+    st_hint(P.stepc + env, done_reset ? 0 : stepc + P.S, l2.state);
     // episode statistics on the device (record_episode_statistics.py:144-171)
     if (P.ep_ret != nullptr) {
       float ep = cur.ep_ret + reward;   // loaded up front with the other inputs
@@ -316,7 +332,7 @@ step_kernel_tile(const __grid_constant__ Params<float> P) {
         atomicAdd(P.ep_acc + 2, 1.0);
         ep = 0.f;
       }
-      P.ep_ret[env] = ep;
+      st_hint(P.ep_ret + env, ep, l2.state);
     }
   }
 
@@ -407,10 +423,10 @@ step_kernel_tile(const __grid_constant__ Params<float> P) {
     for (int i = tid; i < rows * D; i += kBlock) gobs[i] = tile_s[i];
   }
   if (active) {
-    P.s0[g] = make_float4(d.px, d.py, d.pz, d.qx);
-    P.s1[g] = make_float4(d.qy, d.qz, d.qw, d.vx);
-    P.s2[g] = make_float4(d.vy, d.vz, d.wx, d.wy);
-    P.s3[g] = make_float4(d.wz, d.tx, d.ty, d.tz);
+    st_hint(P.s0 + g, make_float4(d.px, d.py, d.pz, d.qx), l2.state);
+    st_hint(P.s1 + g, make_float4(d.qy, d.qz, d.qw, d.vx), l2.state);
+    st_hint(P.s2 + g, make_float4(d.vy, d.vz, d.wx, d.wy), l2.state);
+    st_hint(P.s3 + g, make_float4(d.wz, d.tx, d.ty, d.tz), l2.state);
   }
   // ---- advance the global step count: last CTA out.  Every thread of this CTA consumed
   // gsteps[0] (ring addresses) before the __syncthreads above, so the ticket needs no fence:
