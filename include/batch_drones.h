@@ -237,6 +237,42 @@ int bd_l2_plan(int n_envs, int n_drones, int act_dim, int buf_slots, int track_e
 /* The plan a handle's step kernel runs with (both 0 when the handle does not use the fast tile kernel). */
 int bd_l2_policy(const bd_handle* h, int* keep_state, int* keep_slots);
 
+/* Snapshot of the complete simulator state, for checkpoints that resume mid-episode and for branching / replay from a
+ * state.  An opaque, versioned byte buffer in CALLER-OWNED device memory (256-byte aligned): a 256-byte header (magic,
+ * format version 1, precision, N, M, A, B, plane flags, configuration fingerprint, the bd_get_rng_state 4-tuple, the
+ * bd_episode_stats accumulators), then SoA planes, each starting on a 256-byte boundary, in this order:
+ *   kinematics      4 x Real4[n_total]   (pos, quat, vel, body rates, TARGET_POS)       always
+ *   world ang. vel. Real4[n_total]                                                       BD_SNAP_ANGV (keep_ang_vel)
+ *   controller      13 x Real[n_total]   (9 DSL PID memory + 4 commanded-rpm planes)    BD_SNAP_CTRL (PID / VEL / ONE_D_PID)
+ *   action ring     B x float[n_total][A], by AGE: plane a = the action of a steps ago   always
+ *   step counters   int32[N]                                                             always
+ *   episode returns float[N]                                                             BD_SNAP_EPISODES (track_episodes)
+ * Because the ring is stored by age, a snapshot does not depend on the saving handle's step count.
+ * Restoring needs a handle with the same N, M, task, act_type, drone model, precision, aero flags, integrator,
+ * pyb_freq, ctrl_freq, airframe / controller / spiral constants and episode length (checked against the fingerprint).
+ * Device, seed, auto_reset, reset_mode, action_is_f32, ctrl_reset_on_reset, the L2 plan and BD_PIPELINE may differ, and
+ * so may keep_ang_vel and track_episodes as long as the snapshot carries every plane the target needs (planes the
+ * target has no use for are ignored).  Initial poses and the jitter buffer are configuration, not state: set them with
+ * bd_set_init_poses / bd_set_jitter.  Observations are not part of the snapshot either: the observation of a saved
+ * state is the one the step returned then, and the caller keeps it.
+ * Neither call is capturable (BD_EINVAL while `stream` is capturing); both BD_EINVAL on a poisoned handle. */
+enum { BD_SNAP_ANGV = 1, BD_SNAP_CTRL = 2, BD_SNAP_EPISODES = 4 };
+/* Size in bytes of a snapshot of this shape (host computation only); BD_EINVAL for a malformed shape or flag. */
+int bd_snapshot_layout(int n_envs, int n_drones, int act_dim, int buf_slots, int precision, int flags, int64_t* bytes);
+/* Size of this handle's snapshots (BD_EINVAL for a NULL handle). */
+int64_t bd_snapshot_bytes(const bd_handle* h);
+/* Write the handle's state into snap_dev (bd_snapshot_bytes bytes).  Stream ordered, does not synchronise; a plain
+ * launch, so it runs after the previous step has completed. */
+int bd_save_snapshot(bd_handle* h, void* snap_dev, void* stream);
+/* Restore a snapshot.  Copies the header back, synchronises `stream`, validates it (BD_EINVAL with a message for a bad
+ * magic, version or size, a configuration mismatch or a missing plane), then launches the unpack kernel.
+ *   env_mask_dev == NULL: full restore — every per-env plane, the episode accumulators, and the Philox counter and
+ *     explicit-reset epoch exactly as bd_set_rng_state sets them.  BD_EINVAL once a step was captured into a CUDA graph.
+ *   env_mask_dev (N) uint8: masked restore — only the envs with a non-zero entry; the handle's step count, episode
+ *     accumulators and RNG state are left alone, and the ring is rewritten by age relative to this handle's head.
+ * The next step launch of the handle reads nothing before its dependency wait (DESIGN.md section 4). */
+int bd_load_snapshot(bd_handle* h, const void* snap_dev, const uint8_t* env_mask_dev, void* stream);
+
 int bd_obs_dim(const bd_handle* h);              /* D                                 */
 int bd_act_dim(const bd_handle* h);              /* A                                 */
 int bd_action_buffer_size(const bd_handle* h);   /* B                                 */

@@ -18,12 +18,14 @@ BD_MODEL = {"cf2x": 0, "cf2p": 1, "racer": 2}
 BD_PRECISION = {"fp32": 0, "fp64": 1}
 BD_INTEGRATOR = {"quat": 0, "euler": 1}
 BD_RESET = {"fixed": 0, "jitter_philox": 1, "jitter_buffer": 2}
+BD_SNAP_ANGV, BD_SNAP_CTRL, BD_SNAP_EPISODES = 1, 2, 4   # optional snapshot planes (bd_snapshot_layout)
 
 EXPORTS = (
     "bd_create", "bd_destroy", "bd_set_init_poses", "bd_set_jitter", "bd_reset", "bd_step",
     "bd_step_host", "bd_step_host_compact", "bd_step_many", "bd_set_step_many_mode", "bd_stream_gate", "bd_get_rng_state", "bd_set_rng_state",
     "bd_debug_set_tile_epoch", "bd_l2_plan", "bd_l2_policy", "bd_get_state", "bd_set_state", "bd_get_targets", "bd_episode_stats",
-    "bd_get_controller_state", "bd_set_controller_state", "bd_set_action_f32", "bd_obs_dim", "bd_act_dim",
+    "bd_get_controller_state", "bd_set_controller_state", "bd_set_action_f32",
+    "bd_snapshot_layout", "bd_snapshot_bytes", "bd_save_snapshot", "bd_load_snapshot", "bd_obs_dim", "bd_act_dim",
     "bd_action_buffer_size", "bd_substeps", "bd_launch_count", "bd_last_error", "bd_version",
     "bd_actor_create", "bd_actor_destroy", "bd_actor_set_weights", "bd_actor_forward", "bd_actor_set_trace", "bd_actor_launch_count",
     "bd_actor_last_error", "bd_actor_set_input_norm",
@@ -122,6 +124,14 @@ def load():
     lib.bd_set_controller_state.restype = C.c_int
     lib.bd_set_action_f32.argtypes = [vp, C.c_int]
     lib.bd_set_action_f32.restype = C.c_int
+    lib.bd_snapshot_layout.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int64)]
+    lib.bd_snapshot_layout.restype = C.c_int
+    lib.bd_snapshot_bytes.argtypes = [vp]
+    lib.bd_snapshot_bytes.restype = C.c_int64
+    lib.bd_save_snapshot.argtypes = [vp, vp, vp]
+    lib.bd_save_snapshot.restype = C.c_int
+    lib.bd_load_snapshot.argtypes = [vp, vp, u8p, vp]
+    lib.bd_load_snapshot.restype = C.c_int
     for name in ("bd_obs_dim", "bd_act_dim", "bd_action_buffer_size", "bd_substeps"):
         getattr(lib, name).argtypes = [vp]
         getattr(lib, name).restype = C.c_int

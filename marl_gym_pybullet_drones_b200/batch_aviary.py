@@ -436,6 +436,68 @@ class BatchAviary:
         st = (C.c_uint64 * 4)(*[int(v) for v in state])
         _native.check(self._lib.bd_set_rng_state(self._h, st), "bd_set_rng_state")
 
+    # --------------------------------------------------------------- snapshots
+    @property
+    def snapshot_nbytes(self) -> int:
+        """Bytes of this aviary's snapshots (`bd_snapshot_bytes`)."""
+        self._check_open()
+        return int(self._lib.bd_snapshot_bytes(self._h))
+
+    def snapshot(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The complete simulator state as an opaque uint8 tensor of `snapshot_nbytes` bytes on the aviary's device
+        (`bd_save_snapshot`): drone states, targets, controller memory, action history, step counters, episode
+        returns and accumulators, and the RNG state of the re-spawn draws.  Stream ordered, no host synchronisation.
+        `out`: a contiguous, 256-byte aligned uint8 CUDA tensor of that size to write into."""
+        self._check_open()
+        n = self.snapshot_nbytes
+        if out is None:
+            out = torch.empty(n, dtype=torch.uint8, device=self.device)
+        elif (out.dtype != torch.uint8 or out.numel() != n or not out.is_contiguous() or out.device != self.device
+              or out.data_ptr() % 256):
+            raise ValueError(f"out must be a contiguous, 256-byte aligned uint8 tensor of {n} bytes on {self.device}")
+        _native.check(self._lib.bd_save_snapshot(self._h, C.c_void_p(out.data_ptr()), self._stream()), "bd_save_snapshot")
+        return out
+
+    def restore(self, snap: torch.Tensor, env_mask: Optional[torch.Tensor] = None):
+        """Put the state of `snapshot()` back (`bd_load_snapshot`); `snap` may live on the device or the CPU.
+
+        `env_mask=None` restores everything, the RNG state of the re-spawn draws included: the aviary continues exactly
+        as the one the snapshot was taken from.  With an (N,) bool mask only those envs are restored; the aviary's own
+        RNG state and episode accumulators stay as they are.  The snapshot may come from an aviary with another seed,
+        reset mode, `auto_reset` or device, and from one that keeps more planes (`keep_ang_vel`, `track_episode_stats`)
+        than this one needs; shape, task, physics and constants must match.  Synchronises (the header is checked on
+        the host).  Observations are not written: the observation of a saved state is the one the step returned when
+        it was saved, and the caller keeps it with the snapshot."""
+        self._check_open()
+        snap = torch.as_tensor(snap)
+        if snap.dtype != torch.uint8 or snap.dim() != 1:
+            raise ValueError("[ERROR] in BatchAviary.restore(), snap must be a 1-D uint8 tensor from BatchAviary.snapshot()")
+        if snap.numel() < 256:
+            raise ValueError(f"[ERROR] in BatchAviary.restore(), a snapshot has at least 256 bytes, got {snap.numel()}")
+        want = int(np.frombuffer(snap[:256].cpu().numpy().tobytes()[40:48], dtype=np.int64)[0])   # SnapHeader.bytes
+        if snap.numel() < want:
+            raise ValueError(f"[ERROR] in BatchAviary.restore(), the snapshot buffer holds {snap.numel()} bytes, "
+                             f"its header says {want} (truncated)")
+        temporary = False
+        if snap.device != self.device or not snap.is_contiguous() or snap.data_ptr() % 256:
+            buf = torch.empty(snap.numel(), dtype=torch.uint8, device=self.device)
+            buf.copy_(snap)
+            snap, temporary = buf, True
+        mask_ptr = None
+        if env_mask is not None:
+            m = torch.as_tensor(env_mask)
+            if m.numel() != self.num_envs:
+                raise ValueError(f"[ERROR] in BatchAviary.restore(), env_mask must have {self.num_envs} entries")
+            env_mask = m.to(device=self.device, dtype=torch.uint8).contiguous()
+            temporary = temporary or env_mask.data_ptr() != m.data_ptr()
+            mask_ptr = C.c_void_p(env_mask.data_ptr())
+        rc = self._lib.bd_load_snapshot(self._h, C.c_void_p(snap.data_ptr()), mask_ptr, self._stream())
+        if rc == -1:
+            raise ValueError("[ERROR] in BatchAviary.restore(), " + self._lib.bd_last_error().decode("utf-8", "replace"))
+        _native.check(rc, "bd_load_snapshot")
+        if temporary:   # the unpack kernel reads them: keep them alive until it is done
+            torch.cuda.current_stream(self.device).synchronize()
+
     def _set_action_dtype(self, dtype):
         """fp64 mode: follow the dtype of the actions handed in, like numpy does in the reference
         (float32 actions -> `1 + 0.05*a` is evaluated in float32, BaseRLAviary.py:192)."""

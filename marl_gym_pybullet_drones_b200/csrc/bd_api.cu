@@ -89,6 +89,7 @@ struct bd_handle {
   uint32_t philox_base = 0;    // bd_set_rng_state: offset of the Philox step counter
   int many_mode = 0;           // bd_step_many: 0 = one launch when possible, 1 = always k launches (bd_set_step_many_mode)
   bool poisoned = false;       // a launch failed half-way through a chunked host step: the tile epochs are inconsistent
+  bool restored = false;       // bd_load_snapshot ran since the last step launch: that launch must not prefetch early
   // compact terminal observations (bd_step_host_compact): pinned, device-mapped staging owned by the handle
   int* c_blockcnt = nullptr;   // [blocks of 1024 envs] done envs per block
   int* c_total = nullptr;      // running count of finished envs over the chunks of one step
@@ -116,7 +117,7 @@ void fill_params(const bd_handle* h, bd::Params<R>& P) {
   P.s0 = (R4*)h->s0; P.s1 = (R4*)h->s1; P.s2 = (R4*)h->s2; P.s3 = (R4*)h->s3; P.s4 = (R4*)h->s4;
   P.hist = h->hist; P.stepc = h->stepc; P.gsteps = h->gsteps; P.tile_epoch = h->tile_epoch; P.finished = h->finished;
   P.step_tiles = h->spec.impl == 1 ? (h->cfg.n_envs + 4 * h->EW - 1) / (4 * h->EW) : (h->cfg.n_envs + h->E - 1) / h->E;
-  P.pipeline = h->pipeline; P.pipe_wait = 0; P.early_prefetch = 0; P.ep_ret = h->ep_ret; P.ep_acc = h->ep_acc;
+  P.pipeline = h->pipeline; P.pipe_wait = 0; P.early_prefetch = 1; P.ep_ret = h->ep_ret; P.ep_acc = h->ep_acc;
   P.l2_keep_state = h->l2_keep_state; P.l2_keep_slots = h->l2_keep_slots;
   P.ctrl = (R*)h->ctrl;
   P.act_type = c.act_type; P.ctrl_reset = c.ctrl_reset_on_reset;
@@ -488,11 +489,14 @@ int bd_step(bd_handle* h, const void* actions_dev, float* obs_dev, void* reward_
     P.truncated = truncated_dev;
     P.terminal_obs = terminal_obs_dev;
     P.obs_aligned = (((uintptr_t)obs_dev & 15) == 0) ? 1 : 0;
+    P.early_prefetch = h->restored ? 0 : 1;
     e = bd::launch_step(h->spec, &P, (cudaStream_t)stream);
     P.obs_aligned = 1;
+    P.early_prefetch = 1;
   });
   // the host step count follows the tile epochs the launch will publish: only a launch that was accepted counts
   if (e != cudaSuccess) return fail(BD_ECUDA, "step kernel launch failed: %s", cudaGetErrorString(e));
+  h->restored = false;
   h->launches++;
   h->total_steps++;
   if (h->total_steps >= (long long)h->B * ((1 << 30) / h->B)) {
@@ -658,8 +662,9 @@ int step_host_impl(bd_handle* h, const void* actions_host, float* obs_host, void
         P.truncated = h->h_trunc;
         P.terminal_obs = want_tobs ? h->h_tobs : nullptr;
         P.block0 = b0; P.grid_blocks = b1 - b0; P.advance = (c == chunks - 1) ? 1 : 0;
+        P.early_prefetch = h->restored ? 0 : 1;
         e = bd::launch_step(h->spec, &P, h->hs_a);
-        P.block0 = 0; P.grid_blocks = 0; P.advance = 1;
+        P.block0 = 0; P.grid_blocks = 0; P.advance = 1; P.early_prefetch = 1;
       });
       if (e != cudaSuccess) {
         // chunks 0..c-1 have stepped their tiles and will publish epochs for a step that never completed
@@ -686,6 +691,7 @@ int step_host_impl(bd_handle* h, const void* actions_host, float* obs_host, void
                                 rows * obs_row, cudaMemcpyDeviceToHost, h->hs_b));
     }
     if (e != cudaSuccess) return fail(BD_ECUDA, "step kernel launch failed: %s", cudaGetErrorString(e));
+    h->restored = false;
     h->total_steps++;
     if (h->total_steps >= (long long)h->B * ((1 << 30) / h->B)) {
       h->total_steps = 0;
@@ -780,6 +786,7 @@ int bd_step_many(bd_handle* h, int k, const void* actions_dev, float* obs_dev, v
     e = bd::launch_step_tile_many(h->spec.task, h->spec.act_a, P, k, (long long)(act_step / act_elem), (long long)obs_step, (long long)n,
                                   h->spec, (cudaStream_t)stream);
     if (e != cudaSuccess) return fail(BD_ECUDA, "bd_step_many: kernel launch failed: %s", cudaGetErrorString(e));
+    h->restored = false;   // a plain launch: it started after the unpack kernel had completed
     h->launches++;
     h->total_steps += k;
     return BD_OK;
@@ -955,6 +962,182 @@ int bd_l2_policy(const bd_handle* h, int* keep_state, int* keep_slots) {
   if (!h || !keep_state || !keep_slots) return fail(BD_EINVAL, "bd_l2_policy: null argument");
   *keep_state = h->l2_keep_state;
   *keep_slots = h->l2_keep_slots;
+  return BD_OK;
+}
+
+}  // extern "C"
+
+namespace bd {
+SnapLayout snap_layout(long long n_envs, long long n_drones, int act_dim, int buf_slots, int real_bytes, int flags) {
+  SnapLayout L;
+  const long long n = n_envs * n_drones;
+  long long off = (long long)sizeof(SnapHeader);
+  auto plane = [&](long long bytes) {
+    const long long at = off;
+    off += (bytes + kSnapAlign - 1) / kSnapAlign * kSnapAlign;
+    return at;
+  };
+  for (int k = 0; k < 4; ++k) L.kin[k] = plane(n * 4 * real_bytes);
+  L.angv = (flags & BD_SNAP_ANGV) ? plane(n * 4 * real_bytes) : -1;
+  L.ctrl_stride = (n * real_bytes + kSnapAlign - 1) / kSnapAlign * kSnapAlign;
+  L.ctrl = -1;
+  if (flags & BD_SNAP_CTRL) {
+    L.ctrl = off;
+    off += (long long)kCtrlPlanesHost * L.ctrl_stride;
+  }
+  L.ring_stride = (n * act_dim * 4 + kSnapAlign - 1) / kSnapAlign * kSnapAlign;
+  L.ring = off;
+  off += (long long)buf_slots * L.ring_stride;
+  L.stepc = plane(n_envs * 4);
+  L.ep_ret = (flags & BD_SNAP_EPISODES) ? plane(n_envs * 4) : -1;
+  L.bytes = off;
+  return L;
+}
+}  // namespace bd
+
+namespace {
+
+// FNV-1a over everything a restore needs to match besides N and M (which the header carries in the clear): task,
+// action type, airframe, precision, aero terms, integrator, frequencies, airframe / controller / spiral constants and
+// the episode length.  Seed, reset behaviour, action dtype, L2 plan and the optional planes may differ.
+uint64_t snap_fingerprint(const bd_config& c) {
+  uint64_t f = 1469598103934665603ull;
+  auto mix = [&](const void* p, size_t n) {
+    const unsigned char* b = static_cast<const unsigned char*>(p);
+    for (size_t i = 0; i < n; ++i) { f ^= b[i]; f *= 1099511628211ull; }
+  };
+  const int32_t ints[] = {c.task, c.act_type, c.drone_model, c.precision, c.aero_flags, c.integrator, c.pyb_freq, c.ctrl_freq};
+  mix(ints, sizeof(ints));
+  const double dbl[] = {c.episode_len_sec, c.mass, c.arm, c.kf, c.km, c.ixx, c.iyy, c.izz, c.g, c.thrust2weight,
+                        c.gnd_eff_coeff, c.prop_radius, c.drag_coeff_xy, c.drag_coeff_z, c.dw_coeff_1, c.dw_coeff_2,
+                        c.dw_coeff_3, c.spiral_radius, c.spiral_period, c.height_rate, c.ctrl_mass, c.ctrl_kf, c.speed_limit};
+  mix(dbl, sizeof(dbl));
+  mix(c.prop_xy, sizeof(c.prop_xy));
+  mix(c.target_center, sizeof(c.target_center));
+  return f;
+}
+
+int snap_flags(const bd_handle* h) {
+  return (h->cfg.keep_ang_vel ? BD_SNAP_ANGV : 0) | (h->ctrl ? BD_SNAP_CTRL : 0) | (h->ep_ret ? BD_SNAP_EPISODES : 0);
+}
+
+bd::SnapLayout handle_layout(const bd_handle* h, int flags) {
+  return bd::snap_layout(h->cfg.n_envs, h->cfg.n_drones, h->A, h->B, (int)h->real, flags);
+}
+
+// the checks bd_save_snapshot and bd_load_snapshot share
+int snap_precheck(bd_handle* h, const void* snap, void* stream, const char* what) {
+  if (!h || !snap) return fail(BD_EINVAL, "%s: null argument", what);
+  if ((uintptr_t)snap & (bd::kSnapAlign - 1)) return fail(BD_EINVAL, "%s: the snapshot buffer must be 256-byte aligned", what);
+  if (h->poisoned)
+    return fail(BD_EINVAL, "%s: an earlier launch of this handle failed half-way through a step; destroy the handle", what);
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing((cudaStream_t)stream, &cs) == cudaSuccess && cs != cudaStreamCaptureStatusNone)
+    return fail(BD_EINVAL, "%s: not capturable (the stream is capturing a CUDA graph)", what);
+  return BD_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int bd_snapshot_layout(int n_envs, int n_drones, int act_dim, int buf_slots, int precision, int flags, int64_t* bytes) {
+  if (!bytes) return fail(BD_EINVAL, "bd_snapshot_layout: null output");
+  *bytes = 0;
+  if (n_envs < 1 || n_drones < 1 || n_drones > bd::kMaxDrones || act_dim < 1 || act_dim > 4 || buf_slots < 1)
+    return fail(BD_EINVAL, "bd_snapshot_layout: bad shape");
+  if (precision != BD_F32 && precision != BD_F64) return fail(BD_EINVAL, "bd_snapshot_layout: unknown precision");
+  if (flags & ~(BD_SNAP_ANGV | BD_SNAP_CTRL | BD_SNAP_EPISODES)) return fail(BD_EINVAL, "bd_snapshot_layout: unknown flag");
+  *bytes = bd::snap_layout(n_envs, n_drones, act_dim, buf_slots, precision == BD_F64 ? 8 : 4, flags).bytes;
+  return BD_OK;
+}
+
+int64_t bd_snapshot_bytes(const bd_handle* h) {
+  if (!h) return fail(BD_EINVAL, "bd_snapshot_bytes: null handle");
+  return handle_layout(h, snap_flags(h)).bytes;
+}
+
+int bd_save_snapshot(bd_handle* h, void* snap_dev, void* stream) {
+  int rc = snap_precheck(h, snap_dev, stream, "bd_save_snapshot");
+  if (rc) return rc;
+  DeviceGuard guard(h->cfg.device);
+  const int flags = snap_flags(h);
+  const bd::SnapLayout L = handle_layout(h, flags);
+  bd::SnapHeader hdr;
+  memset(&hdr, 0, sizeof(hdr));
+  hdr.magic = bd::kSnapMagic; hdr.version = bd::kSnapVersion;
+  hdr.precision = h->cfg.precision; hdr.n_envs = h->cfg.n_envs; hdr.n_drones = h->cfg.n_drones;
+  hdr.act_dim = h->A; hdr.buf_slots = h->B; hdr.flags = (uint32_t)flags;
+  hdr.fingerprint = snap_fingerprint(h->cfg);
+  hdr.bytes = L.bytes;
+  bd_get_rng_state(h, hdr.rng);   // rng[1] is recomputed on the device from the step count the ring head uses
+  hdr.task = h->cfg.task; hdr.act_type = h->cfg.act_type; hdr.drone_model = h->cfg.drone_model;
+  hdr.aero_flags = h->cfg.aero_flags; hdr.integrator = h->cfg.integrator;
+  hdr.pyb_freq = h->cfg.pyb_freq; hdr.ctrl_freq = h->cfg.ctrl_freq;
+  // a plain launch (no programmatic serialization): it starts after the previous step has completed
+  cudaError_t e = bd::launch_snapshot(h->cfg.precision, params_ptr(h), snap_dev, L, hdr, nullptr, 1, 0, (cudaStream_t)stream);
+  h->launches++;
+  if (e != cudaSuccess) return fail(BD_ECUDA, "snapshot kernel launch failed: %s", cudaGetErrorString(e));
+  return BD_OK;
+}
+
+int bd_load_snapshot(bd_handle* h, const void* snap_dev, const uint8_t* env_mask_dev, void* stream) {
+  int rc = snap_precheck(h, snap_dev, stream, "bd_load_snapshot");
+  if (rc) return rc;
+  const bool full = env_mask_dev == nullptr;
+  if (full && h->graph_mode)
+    return fail(BD_EINVAL, "bd_load_snapshot: a full restore is not available after a step was captured into a CUDA graph "
+                           "(captured launches carry the Philox offset); restore with an env mask instead");
+  DeviceGuard guard(h->cfg.device);
+  cudaStream_t st = (cudaStream_t)stream;
+  bd::SnapHeader hdr;
+  BD_CUDA(cudaMemcpyAsync(&hdr, snap_dev, sizeof(hdr), cudaMemcpyDeviceToHost, st));
+  BD_CUDA(cudaStreamSynchronize(st));
+  const bd_config& c = h->cfg;
+  if (hdr.magic != bd::kSnapMagic) return fail(BD_EINVAL, "bd_load_snapshot: not a snapshot (bad magic 0x%08x)", hdr.magic);
+  if (hdr.version != bd::kSnapVersion)
+    return fail(BD_EINVAL, "bd_load_snapshot: snapshot format version %u, this library reads version %u", hdr.version,
+                bd::kSnapVersion);
+  if (hdr.precision != BD_F32 && hdr.precision != BD_F64) return fail(BD_EINVAL, "bd_load_snapshot: corrupt header");
+  if (hdr.n_envs != c.n_envs || hdr.n_drones != c.n_drones)
+    return fail(BD_EINVAL, "bd_load_snapshot: the snapshot holds %d envs x %d drones, the handle %d x %d", hdr.n_envs,
+                hdr.n_drones, c.n_envs, c.n_drones);
+  if (hdr.task != c.task) return fail(BD_EINVAL, "bd_load_snapshot: the snapshot is of task %d, the handle of task %d", hdr.task, c.task);
+  if (hdr.act_type != c.act_type)
+    return fail(BD_EINVAL, "bd_load_snapshot: the snapshot has act_type %d, the handle %d", hdr.act_type, c.act_type);
+  if (hdr.precision != c.precision)
+    return fail(BD_EINVAL, "bd_load_snapshot: the snapshot has precision %s, the handle %s", hdr.precision ? "fp64" : "fp32",
+                c.precision ? "fp64" : "fp32");
+  if (hdr.pyb_freq != c.pyb_freq || hdr.ctrl_freq != c.ctrl_freq)
+    return fail(BD_EINVAL, "bd_load_snapshot: the snapshot has pyb_freq %d / ctrl_freq %d, the handle %d / %d", hdr.pyb_freq,
+                hdr.ctrl_freq, c.pyb_freq, c.ctrl_freq);
+  if (hdr.fingerprint != snap_fingerprint(c))
+    return fail(BD_EINVAL, "bd_load_snapshot: the snapshot was taken with a different configuration (drone model, physics, "
+                           "integrator, airframe, controller or spiral constants, or episode length)");
+  if (hdr.act_dim != h->A || hdr.buf_slots != h->B) return fail(BD_EINVAL, "bd_load_snapshot: corrupt header");
+  if (hdr.flags & ~(uint32_t)(BD_SNAP_ANGV | BD_SNAP_CTRL | BD_SNAP_EPISODES))
+    return fail(BD_EINVAL, "bd_load_snapshot: unknown plane flags 0x%x", hdr.flags);
+  const int need = snap_flags(h);
+  if ((need & ~(int)hdr.flags) != 0)
+    return fail(BD_EINVAL, "bd_load_snapshot: the handle needs planes the snapshot lacks (%s%s%s)",
+                (need & ~hdr.flags & BD_SNAP_ANGV) ? "world angular velocity, keep_ang_vel " : "",
+                (need & ~hdr.flags & BD_SNAP_CTRL) ? "controller memory " : "",
+                (need & ~hdr.flags & BD_SNAP_EPISODES) ? "episode returns, track_episodes" : "");
+  const bd::SnapLayout L = handle_layout(h, (int)hdr.flags);
+  if (hdr.bytes != L.bytes)
+    return fail(BD_EINVAL, "bd_load_snapshot: the header says %lld bytes, its layout %lld (truncated or corrupt)",
+                (long long)hdr.bytes, (long long)L.bytes);
+  if (full) {   // exactly what bd_set_rng_state does
+    h->cfg.seed = hdr.rng[0];
+    h->philox_base = (uint32_t)hdr.rng[1] - (uint32_t)h->total_steps;
+    h->reset_epoch = (int)hdr.rng[2];
+    refresh_params(h);
+  }
+  cudaError_t e = bd::launch_snapshot(h->cfg.precision, params_ptr(h), const_cast<void*>(snap_dev), L, hdr, env_mask_dev, 0,
+                                      full ? 1 : 0, st);
+  h->launches++;
+  if (e != cudaSuccess) return fail(BD_ECUDA, "snapshot kernel launch failed: %s", cudaGetErrorString(e));
+  h->restored = true;   // the next step launch must not read ring planes before griddepcontrol.wait
   return BD_OK;
 }
 

@@ -563,6 +563,77 @@ __global__ void set_state_kernel(const __grid_constant__ Params<R> P, const R* k
   }
 }
 
+// Simulator snapshot, both directions (bd_save_snapshot / bd_load_snapshot).  One thread per drone: the four (five)
+// state planes as 128-bit (Real4) accesses, the controller planes, and the B ring slots stored by AGE (age a = ring slot
+// (total-1-a) mod B of this handle), each age plane copied coalesced over drones; threads g < N also carry env g's step
+// counter and episode return.  A masked load touches only the drones / envs with mask[env] != 0.
+template <typename R>
+__global__ void __launch_bounds__(256)
+snapshot_kernel(const __grid_constant__ Params<R> P, unsigned char* snap, const __grid_constant__ SnapLayout L,
+                const __grid_constant__ SnapHeader hdr, const uint8_t* mask, int save, int full) {
+  using R4 = typename V4<R>::type;
+  const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int total = P.host_total >= 0 ? P.host_total : P.gsteps[0];
+  if (g == 0) {
+    SnapHeader* h = reinterpret_cast<SnapHeader*>(snap);
+    if (save) {
+      SnapHeader o = hdr;
+      o.rng[1] = (uint64_t)(uint32_t)(P.philox_base + (uint32_t)total);   // the device count in graph mode
+      for (int k = 0; k < 3; ++k) o.ep_acc[k] = P.ep_acc[k];
+      *h = o;
+    } else if (full) {
+      for (int k = 0; k < 3; ++k) P.ep_acc[k] = h->ep_acc[k];
+    }
+  }
+  if (g < P.N && (save || mask == nullptr || mask[g])) {
+    int* sc = reinterpret_cast<int*>(snap + L.stepc);
+    float* er = L.ep_ret >= 0 ? reinterpret_cast<float*>(snap + L.ep_ret) : nullptr;
+    if (save) {
+      sc[g] = P.stepc[g];
+      if (er != nullptr) er[g] = P.ep_ret[g];
+    } else {
+      P.stepc[g] = sc[g];
+      if (P.ep_ret != nullptr) P.ep_ret[g] = er[g];   // the host refused a snapshot without the plane
+    }
+  }
+  if (g >= P.n_total) return;
+  if (!save && mask != nullptr && !mask[g / P.M]) return;
+  R4* k0 = reinterpret_cast<R4*>(snap + L.kin[0]);
+  R4* k1 = reinterpret_cast<R4*>(snap + L.kin[1]);
+  R4* k2 = reinterpret_cast<R4*>(snap + L.kin[2]);
+  R4* k3 = reinterpret_cast<R4*>(snap + L.kin[3]);
+  R4* av = L.angv >= 0 ? reinterpret_cast<R4*>(snap + L.angv) : nullptr;
+  const int A = P.A, B = P.B;
+  const int newest = (int)(((long long)total + B - 1) % B);
+  if (save) {
+    k0[g] = P.s0[g]; k1[g] = P.s1[g]; k2[g] = P.s2[g]; k3[g] = P.s3[g];
+    if (av != nullptr) av[g] = P.s4[g];
+  } else {
+    P.s0[g] = k0[g]; P.s1[g] = k1[g]; P.s2[g] = k2[g]; P.s3[g] = k3[g];
+    if (P.keep_angv) P.s4[g] = av[g];
+  }
+  if (P.ctrl != nullptr) {
+    for (int k = 0; k < kCtrlPlanesHost; ++k) {
+      R* c = reinterpret_cast<R*>(snap + L.ctrl + k * L.ctrl_stride);
+      R* s = P.ctrl + (size_t)k * P.n_total;
+      if (save) c[g] = s[g]; else s[g] = c[g];
+    }
+  }
+  for (int a = 0; a < B; ++a) {
+    int slot = newest - a;
+    if (slot < 0) slot += B;
+    float* hs = P.hist + ((size_t)slot * P.n_total + g) * A;
+    float* rs = reinterpret_cast<float*>(snap + L.ring + a * L.ring_stride) + g * A;
+    const float* src = save ? hs : rs;
+    float* dst = save ? rs : hs;
+    if (A == 4) {
+      *reinterpret_cast<float4*>(dst) = *reinterpret_cast<const float4*>(src);
+    } else {
+      for (int k = 0; k < A; ++k) dst[k] = src[k];
+    }
+  }
+}
+
 // DSL PID memory (N,M,9): [integral_pos_e, integral_rpy_e, last_rpy]; src == nullptr zeroes it
 // (DSLPIDControl.reset, DSLPIDControl.py:64-79)
 template <typename R>
@@ -728,6 +799,19 @@ cudaError_t launch_ctrl_state(int precision, const void* p, void* dst, const voi
   } else {
     const auto& P = *static_cast<const Params<float>*>(p);
     ctrl_state_kernel<float><<<flat_grid(P), 256, 0, st>>>(P, (float*)dst, (const float*)src, write);
+  }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_snapshot(int precision, const void* p, void* snap, const SnapLayout& L, const SnapHeader& hdr,
+                            const uint8_t* mask, int save, int full, cudaStream_t st) {
+  unsigned char* s = static_cast<unsigned char*>(snap);
+  if (precision) {
+    const auto& P = *static_cast<const Params<double>*>(p);
+    snapshot_kernel<double><<<flat_grid(P), 256, 0, st>>>(P, s, L, hdr, mask, save, full);
+  } else {
+    const auto& P = *static_cast<const Params<float>*>(p);
+    snapshot_kernel<float><<<flat_grid(P), 256, 0, st>>>(P, s, L, hdr, mask, save, full);
   }
   return cudaGetLastError();
 }

@@ -69,7 +69,9 @@ struct Params {
   long long step_tiles;           // tiles of one whole control step with this handle's kernel
   int pipeline;                   // 1: the handle pipelines steps tile by tile: every launch publishes tile epochs
   int pipe_wait;                  // 1: this launch waits for MY tile's previous step only (no grid-wide dependency wait)
-  int early_prefetch;             // 1: ring planes may be prefetched before griddepcontrol.wait (grid >= resident capacity)
+  int early_prefetch;             // 1: ring planes may be prefetched before griddepcontrol.wait (grid >= resident capacity).
+                                  // Host side 0 forbids it for one launch (the first step after bd_load_snapshot, whose
+                                  // unpack kernel wrote those planes); launch_step_tile decides the value the kernel sees
   int block0, grid_blocks;        // sub-range launch: first tile and tile count (0 = all tiles)
   int advance;                    // 1: this launch advances the device-resident step count (last chunk of a step)
   int reset_epoch;                // >=1 for explicit bd_reset calls (Philox stream id), 0 in-step
@@ -81,6 +83,31 @@ struct Params {
   int l2_keep_state;
   int l2_keep_slots;
 };
+
+// Simulator snapshot (bd_save_snapshot / bd_load_snapshot, include/batch_drones.h): a 256-byte header, then SoA planes,
+// each starting on a 256-byte boundary, in this order: s0..s3, [s4], [13 controller planes], B ring planes by age,
+// step counters, [episode returns].
+constexpr uint32_t kSnapMagic = 0x4e534442u;   // "BDSN"
+constexpr uint32_t kSnapVersion = 1;
+constexpr long long kSnapAlign = 256;
+struct SnapHeader {
+  uint32_t magic, version;
+  int32_t precision, n_envs, n_drones, act_dim, buf_slots;
+  uint32_t flags;                 // BD_SNAP_* planes present
+  uint64_t fingerprint;           // configuration that must match on restore (bd_api.cu: snap_fingerprint)
+  int64_t bytes;                  // whole snapshot, header included
+  uint64_t rng[4];                // bd_get_rng_state of the saving handle
+  double ep_acc[3];               // episode accumulators (bd_episode_stats)
+  int32_t task, act_type, drone_model, aero_flags, integrator, pyb_freq, ctrl_freq, reserved0;
+  uint8_t reserved[120];
+};
+static_assert(sizeof(SnapHeader) == 256, "snapshot header is 256 bytes");
+// byte offsets of the planes; -1 = not present
+struct SnapLayout {
+  long long kin[4], angv, ctrl, ctrl_stride, ring, ring_stride, stepc, ep_ret, bytes;
+};
+// host computation shared by bd_snapshot_layout and the handle calls (bd_api.cu)
+SnapLayout snap_layout(long long n_envs, long long n_drones, int act_dim, int buf_slots, int real_bytes, int flags);
 
 struct LaunchSpec {
   int task, act_a, precision, generic, device;
@@ -105,6 +132,10 @@ cudaError_t launch_get_targets(int precision, const void* params, void* targets,
 cudaError_t launch_ctrl_state(int precision, const void* params, void* dst, const void* src, int write,
                               cudaStream_t st);
 cudaError_t launch_episode_stats(double* ep_acc, double* out3, int reset, cudaStream_t st);
+// save = 1: state -> snapshot (header written from `hdr`, ep_acc and the Philox counter filled in on the device);
+// save = 0: snapshot -> state for the envs with mask[e] != 0 (all when NULL); full = 1 also restores ep_acc
+cudaError_t launch_snapshot(int precision, const void* params, void* snap, const SnapLayout& L, const SnapHeader& hdr,
+                            const uint8_t* mask, int save, int full, cudaStream_t st);
 size_t step_smem_bytes(int precision, int A, int B, int D, int task);
 int compact_blocks(int n);
 cudaError_t launch_compact_done(const uint8_t* term, const uint8_t* trunc, int e0, int e1, int reset_total, int* blockcnt, int* total,

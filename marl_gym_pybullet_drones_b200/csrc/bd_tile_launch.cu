@@ -38,7 +38,11 @@ static cudaError_t launch_step_tile_t(const Params<float>& P, const LaunchSpec& 
     per_sm_smem[(vecrow ? 1 : 0) + 2 * aero][dv] = smem;
   }
   Params<float> Q = P;
-  Q.early_prefetch = (ls.pdl && grid >= occ * ls.sm_count) ? 1 : 0;
+  // P.early_prefetch == 0: the launch right after bd_load_snapshot.  Its programmatic primary is the unpack kernel, which
+  // wrote every ring plane, so nothing may be read before griddepcontrol.wait.  (With pipe_wait the kernel takes the
+  // pipe_gate branch instead: the restore synchronised the stream, the finished-tile counter shows the previous step
+  // complete, and every CTA executes griddepcontrol.wait before its first load.)
+  Q.early_prefetch = (P.early_prefetch && ls.pdl && grid >= occ * ls.sm_count) ? 1 : 0;
   Q.pipe_wait = (P.pipeline && ls.pdl && grid >= occ * ls.sm_count) ? 1 : 0;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);

@@ -75,6 +75,8 @@ MAPPO_CONFIG = {   # reference mappo/config.py:3-48 with the learn_mappo.py:179-
     "norm_reward": False,
     "clip_obs": 10,
     "clip_reward": 10,
+    "save_env_state": False,      # state_dict() also stores the simulator snapshot and the rollout loop's state under
+                                  # "resume", so a resumed run continues mid-episode instead of resetting every env
 }
 
 
@@ -216,6 +218,7 @@ class DeviceMAPPO:
         # (the step kernel accumulates them: BatchAviary.episode_stats)
         self.total_env_steps = 0
         self._reset_done = False
+        self._resumed = False     # obs[0] holds the observation a checkpoint's "resume" block restored
         self.fused = None
         if self.cfg["fused_actor"] and self.cfg["activation"] == "tanh":
             from ._native import NativeError
@@ -268,6 +271,8 @@ class DeviceMAPPO:
         """T env steps for all N envs; no host synchronisation inside the loop."""
         if not self._reset_done:
             self.reset()
+        elif self._resumed:
+            self._resumed = False                 # obs[0] and its statistics came from the checkpoint
         elif self.total_env_steps > 0:
             self.obs[0].copy_(self.obs[self.T])   # the rollout continues where the previous one stopped
             if self.norm_obs:
@@ -614,7 +619,9 @@ class DeviceMAPPO:
     def state_dict(self):
         """The reference's checkpoint layout (`MAPPO.save`, mappo/mappo.py:203-232): `agent` =
         {`ac` with the reference's parameter names, `actor_opt`, `critic_opt`}, `obs_normalizer`,
-        `reward_normalizer`, `total_steps`, `obs` (the current, normalised observation)."""
+        `reward_normalizer`, `total_steps`, `obs` (the current, normalised observation).  With
+        `save_env_state=True` one more key, `resume`, carries the simulator snapshot and the rollout loop's state
+        (`_resume_state`); `load_state_dict` applies it whenever it is present."""
         sd = {"agent": {"ac": self.ac.reference_state_dict(), "actor_opt": self.actor_opt.state_dict(),
                         "critic_opt": self.critic_opt.state_dict()},
               "obs_normalizer": self.obs_normalizer.state_dict(),
@@ -624,10 +631,71 @@ class DeviceMAPPO:
               "random_state": {"torch_generator": self.gen.get_state().cpu(),
                                "fused_calls": int(self.fused._calls) if self.fused is not None else 0},
               "env_random_state": [{"philox": self.env.get_rng_state()}]}
+        t = self._current_slot()
         if self._reset_done:
-            t = self.T if self.total_env_steps > 0 else 0
             sd["obs"] = self._normed(self.obs[t], t).cpu().numpy()
+        if self.cfg["save_env_state"]:
+            sd["resume"] = self._resume_state(t)
         return sd
+
+    def _current_slot(self):
+        """Rollout slot holding the observation the next rollout starts from."""
+        return self.T if self.total_env_steps > 0 and not self._resumed else 0
+
+    def _shard(self):
+        """(rank, world, env offset, env count) of this process's env shard; collective when world > 1."""
+        rank = torch.distributed.get_rank() if torch.distributed.is_initialized() else 0
+        offset = 0
+        if self._world > 1:
+            counts = torch.zeros(self._world, dtype=torch.int64, device=self.device)
+            torch.distributed.all_gather_into_tensor(counts, torch.tensor([self.N], dtype=torch.int64, device=self.device))
+            offset = int(counts[:rank].sum())
+        return rank, self._world, offset, self.N
+
+    def _resume_state(self, t):
+        """What `load_state_dict` needs besides the reference-layout keys to continue mid-episode: the simulator
+        snapshot, the raw observation slot the next rollout starts from (with its normaliser statistics), the
+        normalisers' internals and the fused actor's noise seed.  With several ranks every rank saves its own shard."""
+        rank, world, offset, count = self._shard()
+        res = {"env": self.env.snapshot().cpu(), "rank": rank, "world": world, "env_offset": offset, "env_count": count,
+               "reset_done": self._reset_done, "fused_seed": int(self._fused_seed)}
+        if self._reset_done and self.norm_obs:   # without norm_obs, sd["obs"] already is the raw slot
+            res["obs"] = self.obs[t].cpu()
+            res["nmean"], res["nrstd"] = self.nmean[t].cpu(), self.nrstd[t].cpu()
+        if self.norm_obs:
+            res["obs_count"] = self.obs_normalizer.rms.count
+        rn = self.reward_normalizer
+        if isinstance(getattr(rn, "count", None), torch.Tensor):
+            res["reward_count"] = rn.count.cpu()
+            res["reward_ret"] = rn.ret.cpu() if rn.ret is not None else None
+        return res
+
+    def _load_resume(self, res, sd):
+        rank, world, offset, count = self._shard()
+        got = (res.get("rank"), res.get("world"), res.get("env_offset"), res.get("env_count"))
+        if got != (rank, world, offset, count):
+            raise ValueError(f"[ERROR] in DeviceMAPPO.load(), the checkpoint's env state belongs to rank {got[0]} of "
+                             f"{got[1]} (envs {got[2]}..{got[2] + got[3] - 1 if got[3] else '?'}); this process is rank "
+                             f"{rank} of {world} (envs {offset}..{offset + count - 1}). Re-sharding is not supported")
+        if self.norm_obs and res.get("reset_done") and "nmean" not in res:
+            raise ValueError("[ERROR] in DeviceMAPPO.load(), the checkpoint was saved without norm_obs")
+        self.env.restore(res["env"])
+        if res.get("reset_done"):
+            raw = res["obs"] if "obs" in res else sd["obs"]
+            self.obs[0].copy_(torch.as_tensor(raw).to(self.device))
+            if self.norm_obs:
+                self.nmean[0].copy_(res["nmean"].to(self.device))
+                self.nrstd[0].copy_(res["nrstd"].to(self.device))
+            self._reset_done = self._resumed = True
+        else:
+            self._reset_done = self._resumed = False
+        if self.norm_obs and "obs_count" in res:
+            self.obs_normalizer.rms.set(count=res["obs_count"])
+        rn = self.reward_normalizer
+        if "reward_count" in res and isinstance(getattr(rn, "count", None), torch.Tensor):
+            rn.count = res["reward_count"].to(self.device)
+            rn.ret = res["reward_ret"].to(self.device) if res["reward_ret"] is not None else None
+        self._fused_seed = int(res["fused_seed"])
 
     def load_state_dict(self, sd):
         self.ac.load_reference_state_dict(sd["agent"]["ac"])
@@ -646,6 +714,8 @@ class DeviceMAPPO:
         ers = sd.get("env_random_state")
         if ers and isinstance(ers[0], dict) and "philox" in ers[0]:
             self.env.set_rng_state(ers[0]["philox"])
+        if sd.get("resume") is not None:   # saved with save_env_state=True: continue mid-episode
+            self._load_resume(sd["resume"], sd)
         self._fused_stale = True
         self._graph = None          # captured graphs have the old hyper-parameters (lr, betas) baked in
         self._pack_native()
