@@ -399,12 +399,6 @@ int bd_ppo_adv_stats(const double* acc3_dev, float* stats2_dev, void* stream);
 /* diagnostics: CTA 0 of the following forward / sample launches writes SM-clock stamps of its pipeline phases
  * ([tile pair][64] int64, see csrc/bd_ppo.cu); NULL switches tracing off */
 int bd_ppo_set_trace(bd_ppo_net* n, long long* trace_dev);
-/* which forward / loss / backward kernel bd_ppo_grad launches: 0 (default) one 128-row tile in flight per CTA, 1 two tiles in
- * flight (one in-place activation buffer per tile, every weight slab serving both tiles); same results */
-int bd_ppo_set_train_mode(bd_ppo_net* n, int mode);
-/* which kernel bd_ppo_forward / bd_ppo_sample launch for an actor net: 0 (default) two tiles in flight per CTA, weights
- * streamed from L2; 1 the CTA-pair kernel (cta_group::2: M = 256 MMAs, half of every weight matrix resident per CTA) */
-int bd_ppo_set_forward_mode(bd_ppo_net* n, int mode);
 int64_t bd_ppo_launch_count(const bd_ppo_net* n);
 const char* bd_ppo_last_error(void);
 

@@ -31,7 +31,7 @@ EXPORTS = (
     "bd_actor_last_error", "bd_actor_set_input_norm",
     "bd_rms_create", "bd_rms_destroy", "bd_rms_update", "bd_rms_batch_moments", "bd_rms_merge_moments", "bd_rms_normalize", "bd_rms_get", "bd_rms_set",
     "bd_rms_launch_count", "bd_rms_last_error",
-    "bd_ppo_net_create", "bd_ppo_net_destroy", "bd_ppo_net_param_count", "bd_ppo_net_stats", "bd_ppo_net_pack", "bd_ppo_forward", "bd_ppo_sample", "bd_ppo_set_trace", "bd_ppo_set_train_mode", "bd_ppo_set_forward_mode",
+    "bd_ppo_net_create", "bd_ppo_net_destroy", "bd_ppo_net_param_count", "bd_ppo_net_stats", "bd_ppo_net_pack", "bd_ppo_forward", "bd_ppo_sample", "bd_ppo_set_trace",
     "bd_ppo_grad", "bd_ppo_adam_step", "bd_ppo_gae", "bd_ppo_adv_stats", "bd_ppo_launch_count", "bd_ppo_last_error",
     "bd_peer_create", "bd_peer_destroy", "bd_peer_handle_size", "bd_peer_get_handle", "bd_peer_open", "bd_peer_data", "bd_peer_allreduce",
     "bd_peer_unmap", "bd_peer_launch_count", "bd_peer_last_error",
@@ -198,10 +198,6 @@ def load():
     lib.bd_ppo_sample.restype = C.c_int
     lib.bd_ppo_set_trace.argtypes = [vp, vp]
     lib.bd_ppo_set_trace.restype = C.c_int
-    lib.bd_ppo_set_train_mode.argtypes = [vp, C.c_int]
-    lib.bd_ppo_set_train_mode.restype = C.c_int
-    lib.bd_ppo_set_forward_mode.argtypes = [vp, C.c_int]
-    lib.bd_ppo_set_forward_mode.restype = C.c_int
     lib.bd_ppo_grad.argtypes = [vp, C.c_int, vp, C.c_int, C.c_int, vp, C.c_int64, vp, vp, vp, vp, vp, vp, C.c_float, C.c_int,
                                 C.c_float, vp, vp, C.c_float, C.c_int64, vp, vp, vp]
     lib.bd_ppo_grad.restype = C.c_int

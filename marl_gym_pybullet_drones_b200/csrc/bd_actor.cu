@@ -119,16 +119,6 @@ struct ActorDev {
   long long* trace;   // optional: [tiles of CTA 0][16] SM-clock stamps of the pipeline phases (bd_actor_set_trace)
 };
 
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t v[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,"
-      "%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-        "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-        "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr));
-}
 __device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t v[16]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
@@ -136,13 +126,11 @@ __device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t v[16])
         "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
       : "r"(taddr));
 }
-template <int CW>
-__device__ __forceinline__ void tmem_ld_nowait(uint32_t taddr, uint32_t* v) {
-  if constexpr (CW == 32) tmem_ld32_nowait(taddr, v); else tmem_ld16_nowait(taddr, v);
-}
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-template <int HID, int CW>
+constexpr int CW = 16;   // columns per TMEM load / published chunk of a hidden epilogue
+
+template <int HID>
 __device__ __forceinline__ void hidden_chunk(const uint32_t* v, int c0, const float* __restrict__ bias, __nv_bfloat16* sH, int row) {
 #pragma unroll
   for (int q = 0; q < CW / 8; ++q) {
@@ -190,30 +178,30 @@ __device__ __forceinline__ void bulk_g2s(uint32_t sdst, const void* gsrc, uint32
                : "memory");
 }
 
-// TMEM accumulator row -> +bias, tanh -> bf16 activation tile (next layer's A operand), 32 columns
+// TMEM accumulator row -> +bias, tanh -> bf16 activation tile (next layer's A operand), 16 columns
 // at a time.  After each chunk the thread publishes it (generic -> async proxy fence, mbarrier
 // arrive): the MMA warp starts the next layer's K-steps over those columns while the remaining
 // chunks are still going through the SFU, so tensor pipe and epilogue overlap inside one tile.
-// The TMEM read of the next 32 columns is in flight while the current 32 are processed.
-template <int HID, int CW>
+// The TMEM read of the next 16 columns is in flight while the current 16 are processed.
+template <int HID>
 __device__ __forceinline__ void epilogue_hidden(uint32_t tmem_row, const float* __restrict__ bias, __nv_bfloat16* sH, int row,
                                                 int cbeg, int n_chunks, uint32_t chunk_bar0) {
   uint32_t va[CW], vb[CW];
-  tmem_ld_nowait<CW>(tmem_row + (uint32_t)cbeg, va);
+  tmem_ld16_nowait(tmem_row + (uint32_t)cbeg, va);
   tmem_wait_ld();
 #pragma unroll 1
   for (int j = 0; j < n_chunks; j += 2) {
     const int c0 = cbeg + j * CW;
     const bool more1 = j + 1 < n_chunks;
-    if (more1) tmem_ld_nowait<CW>(tmem_row + (uint32_t)(c0 + CW), vb);
-    hidden_chunk<HID, CW>(va, c0, bias, sH, row);
+    if (more1) tmem_ld16_nowait(tmem_row + (uint32_t)(c0 + CW), vb);
+    hidden_chunk<HID>(va, c0, bias, sH, row);
     proxy_fence();
     mbar_arrive(chunk_bar0 + 8u * (uint32_t)j);
     tmem_wait_ld();
     if (!more1) break;
     const bool more2 = j + 2 < n_chunks;
-    if (more2) tmem_ld_nowait<CW>(tmem_row + (uint32_t)(c0 + 2 * CW), va);
-    hidden_chunk<HID, CW>(vb, c0 + CW, bias, sH, row);
+    if (more2) tmem_ld16_nowait(tmem_row + (uint32_t)(c0 + 2 * CW), va);
+    hidden_chunk<HID>(vb, c0 + CW, bias, sH, row);
     proxy_fence();
     mbar_arrive(chunk_bar0 + 8u * (uint32_t)(j + 1));
     tmem_wait_ld();
@@ -225,21 +213,22 @@ constexpr int kMaxChunks = 4;                 // column chunks per thread and la
 enum { BAR_STAGE = 0, BAR_L1, BAR_L2, BAR_L3, BAR_W1, BAR_W23, BAR_H1, BAR_H2 = BAR_H1 + kMaxChunks,
        BAR_COUNT = BAR_H2 + kMaxChunks };
 
-// G = threads per row (column groups): warps 0..4G-1 stage and run the epilogues (warp w owns TMEM
+// G = 4 threads per row (column groups): warps 0..4G-1 stage and run the epilogues (warp w owns TMEM
 // lanes 32*(w%4).. and column group w/4), warp 4G issues every tcgen05.mma and TMA copy.
-// G = 4 (16 epilogue warps, 4 per SM sub-partition) hides the TMEM-load / MUFU latencies of the
-// tanh epilogue twice as well as G = 2; the register file then allows 96 registers per thread.
-template <int G> struct ActorShape {
+// 16 epilogue warps (4 per SM sub-partition) hide the TMEM-load / MUFU latencies of the tanh
+// epilogue twice as well as G = 2 did; the register file then allows 96 registers per thread.
+struct ActorShape {
+  static constexpr int G = 4;
   static constexpr int kEpiThreads = kRows * G;
   static constexpr int kThreads = kEpiThreads + 32;
 };
 
-template <int HID, int G>
-__global__ void __launch_bounds__(ActorShape<G>::kThreads, 1)
+template <int HID>
+__global__ void __launch_bounds__(ActorShape::kThreads, 1)
 actor_forward_kernel(ActorDev W, const float* __restrict__ obs, long long rows, const float* __restrict__ noise,
                      unsigned long long seed, unsigned long long offset, float* __restrict__ act, float* __restrict__ logp,
                      float* __restrict__ mean_out) {
-  constexpr int kEpiThreads = ActorShape<G>::kEpiThreads, kThreads = ActorShape<G>::kThreads;
+  constexpr int G = ActorShape::G, kEpiThreads = ActorShape::kEpiThreads, kThreads = ActorShape::kThreads;
   extern __shared__ __align__(128) unsigned char smem[];
   const int K1 = W.K1;
   const size_t actb = (size_t)kRows * HID * 2, l1b = (size_t)(kRows + HID) * K1 * 2;
@@ -260,7 +249,6 @@ actor_forward_kernel(ActorDev W, const float* __restrict__ obs, long long rows, 
   const int row = tid & (kRows - 1);      // my row of the tile = my TMEM lane
   const int grp = (tid >> 7) & (G - 1);   // which group of columns I handle in the epilogues
   constexpr int kGrpCols = HID / G;       // columns per thread and layer
-  constexpr int CW = (G == 2 && kGrpCols >= 32) ? 32 : 16;   // columns per TMEM load / published chunk
   constexpr int kChunks = kGrpCols / CW;
   static_assert(kChunks >= 1 && kChunks <= kMaxChunks, "unsupported HID / G");
   constexpr uint32_t kTmemCols = HID == 256 ? 512u : (HID == 128 ? 256u : 128u);   // two accumulators
@@ -467,14 +455,14 @@ actor_forward_kernel(ActorDev W, const float* __restrict__ obs, long long rows, 
       mbar_wait_guarded(bar(BAR_L1), parity);
       tc_fence_after();
       if (tr) tr[1] = clock64();      // layer-1 accumulator ready
-      epilogue_hidden<HID, CW>(acc0 + lane_off, sB1, sA, row, cbeg, kChunks, bar(BAR_H1));
+      epilogue_hidden<HID>(acc0 + lane_off, sB1, sA, row, cbeg, kChunks, bar(BAR_H1));
       tc_fence_before();
       if (tr) tr[2] = clock64();      // my layer-1 epilogue done
       // ---- layer-2 epilogue: H2 over H1 (layer-2 MMAs are complete), chunks feed layer 3 -------------
       mbar_wait_guarded(bar(BAR_L2), parity);
       tc_fence_after();
       if (tr) tr[3] = clock64();      // layer-2 accumulator ready
-      epilogue_hidden<HID, CW>(acc1 + lane_off, sB2, sA, row, cbeg, kChunks, bar(BAR_H2));
+      epilogue_hidden<HID>(acc1 + lane_off, sB2, sA, row, cbeg, kChunks, bar(BAR_H2));
       tc_fence_before();
       if (tr) tr[4] = clock64();      // my layer-2 epilogue done
       // ---- layer 3 done: pull my row's 16 outputs out of TMEM, hand region A and acc0 to the next
@@ -1003,14 +991,12 @@ __global__ void pad_vector_kernel(const float* __restrict__ v, int n, int n_pad,
 
 using ActorKernel = void (*)(ActorDev, const float*, long long, const float*, unsigned long long, unsigned long long, float*,
                              float*, float*);
-static ActorKernel actor_kernel(int hidden, int groups) {
-  if (groups == 2) return hidden == 256 ? actor_forward_kernel<256, 2> : (hidden == 128 ? actor_forward_kernel<128, 2> : actor_forward_kernel<64, 2>);
-  return hidden == 256 ? actor_forward_kernel<256, 4> : (hidden == 128 ? actor_forward_kernel<128, 4> : actor_forward_kernel<64, 4>);
+static ActorKernel actor_kernel(int hidden) {
+  return hidden == 256 ? actor_forward_kernel<256> : (hidden == 128 ? actor_forward_kernel<128> : actor_forward_kernel<64>);
 }
 
 struct bd_actor {
   int device, obs_dim, hidden, act_dim, K1, sm_count;
-  int groups = 4;   // threads per row in the epilogues (BD_ACTOR_GROUPS=2 selects the 8-warp variant)
   __nv_bfloat16 *w1 = nullptr, *w2 = nullptr, *w3 = nullptr;
   float *b1 = nullptr, *b2 = nullptr, *b3 = nullptr, *logstd = nullptr;
   size_t smem = 0;
@@ -1053,14 +1039,11 @@ int bd_actor_create(int obs_dim, int hidden, int act_dim, int device, bd_actor**
   alloc((void**)&a->w3, (size_t)kNOut * hidden * 2);
   alloc((void**)&a->b1, hidden * 4); alloc((void**)&a->b2, hidden * 4);
   alloc((void**)&a->b3, kNOut * 4); alloc((void**)&a->logstd, kNOut * 4);
-  if (hidden == 256) {   // TMEM-resident variant: W1 / W2 / W3 resident + one or two observation tiles (BD_ACTOR_IMPL=smem opts out)
+  if (hidden == 256) {   // TMEM-resident variant: W1 / W2 / W3 resident + one or two observation tiles
     const size_t fixed = (size_t)(hidden * K1 + hidden * hidden) * 2 + (size_t)(2 * hidden + 2 * kNOut) * 4 + (size_t)(hidden + 4 * kRows) * 16;
     const size_t xb = (size_t)kRows * K1 * 2, room = prop.sharedMemPerBlockOptin - 1024;   // static shared memory: barriers
-    const char* im = getenv("BD_ACTOR_IMPL");
-    if (!(im && im[0] == 's')) {
-      if (fixed + 2 * xb <= room) { a->impl = 2; a->smem_t = fixed + 2 * xb; }
-      else if (fixed + xb <= room) { a->impl = 1; a->smem_t = fixed + xb; }
-    }
+    if (fixed + 2 * xb <= room) { a->impl = 2; a->smem_t = fixed + 2 * xb; }
+    else if (fixed + xb <= room) { a->impl = 1; a->smem_t = fixed + xb; }
   }
   if (a->impl == 0 && a->smem > prop.sharedMemPerBlockOptin) {
     cudaFree(a->w1); cudaFree(a->w2); cudaFree(a->w3); cudaFree(a->b1); cudaFree(a->b2); cudaFree(a->b3); cudaFree(a->logstd);
@@ -1071,10 +1054,8 @@ int bd_actor_create(int obs_dim, int hidden, int act_dim, int device, bd_actor**
                  need, (size_t)prop.sharedMemPerBlockOptin);
   }
   if (e == cudaSuccess) {
-    const char* g = getenv("BD_ACTOR_GROUPS");
-    if (g && g[0] == '2') a->groups = 2;
     if (a->impl == 0)
-      e = cudaFuncSetAttribute(actor_kernel(hidden, a->groups), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)a->smem);
+      e = cudaFuncSetAttribute(actor_kernel(hidden), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)a->smem);
     else
       e = cudaFuncSetAttribute(a->impl == 2 ? actor_tmem_kernel<2> : actor_tmem_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                (int)a->smem_t);
@@ -1127,9 +1108,8 @@ int bd_actor_forward(bd_actor* a, const float* obs_dev, int64_t rows, const floa
     (a->impl == 2 ? actor_tmem_kernel<2> : actor_tmem_kernel<1>)<<<grid, kTThreads, a->smem_t, st>>>(W, obs_dev, rows, noise_dev, seed,
                                                                                                    offset, act_dev, logp_dev, mean_dev);
   } else {
-    const int threads = a->groups == 2 ? ActorShape<2>::kThreads : ActorShape<4>::kThreads;
-    actor_kernel(a->hidden, a->groups)<<<grid, threads, a->smem, st>>>(W, obs_dev, rows, noise_dev, seed, offset, act_dev, logp_dev,
-                                                                      mean_dev);
+    actor_kernel(a->hidden)<<<grid, ActorShape::kThreads, a->smem, st>>>(W, obs_dev, rows, noise_dev, seed, offset, act_dev, logp_dev,
+                                                                        mean_dev);
   }
   a->launches++;
   cudaError_t e = cudaGetLastError();

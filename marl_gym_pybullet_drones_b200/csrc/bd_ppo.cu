@@ -128,13 +128,10 @@ struct NetDev {
   const bf16* w3b_slab;    // [256 j x 16 o] = W3[o][j]
   const float *b1, *b2, *b3, *logstd;   // b3 / logstd padded to 16
   int C, D, K1p, out_dim;
-  // CTA-pair kernel (actor nets, C == 1): per cluster rank r the N-half of every weight, resident in that CTA's shared
-  // memory: w1c [2][128 n x K1p], w2c [2][128 n x 256], w3c [2][8 n x 256], canonical K-major
-  const bf16 *w1c, *w2c, *w3c;
 };
 
 
-enum { MODE_ACTOR_TRAIN = 0, MODE_CRITIC_TRAIN = 1, MODE_FORWARD = 2 };
+enum { MODE_ACTOR_TRAIN = 0, MODE_CRITIC_TRAIN = 1 };
 
 struct TileArgs {
   NetDev net;
@@ -149,7 +146,6 @@ struct TileArgs {
   const float *nmean, *nrstd;   // optional observation normalisation: per slot (t), per (agent, column)
   float nclip;
   bf16 *Xt, *H1t, *H2t, *dZ2t, *dZ1t, *dZ3t;   // tile scratch for dw_kernel
-  float* out;                // MODE_FORWARD: (rows, out_dim)
   double* stats;             // [0] sum loss, [1] sum (logp_old - logp), [2] rows, [3..6] dlogstd sums, [7..10] db3 sums
   int stages;                // ring depth (<= kMaxStages)
   long long* trace;          // diagnostics: CTA 0's epilogue thread 0 writes [tile][16] SM-clock stamps of its phases
@@ -182,7 +178,6 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
   __shared__ float s_red[11];   // CTA-wide sums of the tiles' statistics, flushed to P.stats once at the end
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const bool train = P.mode != MODE_FORWARD;
   for (int i = tid; i < HID; i += kThreads) { sB1[i] = W.b1[i]; sB2[i] = W.b2[i]; }
   if (tid < kNOut) { sB3[tid] = W.b3[tid]; sLs[tid] = W.logstd != nullptr ? W.logstd[tid] : 0.f; }
   if (tid < 11) s_red[tid] = 0.f;
@@ -236,11 +231,9 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
         for (int q = 0; q < n1; ++q) push(W.w1_slabs + (size_t)q * (kSlabBytes / 2));
 #pragma unroll 4
         for (int q = 0; q < 16; ++q) push(W.w2f_slabs + (size_t)q * (kSlabBytes / 2));
-        if (train) {
-          push(W.w3b_slab);
+        push(W.w3b_slab);
 #pragma unroll 4
-          for (int q = 0; q < 16; ++q) push(W.w2b_slabs + (size_t)q * (kSlabBytes / 2));
-        }
+        for (int q = 0; q < 16; ++q) push(W.w2b_slabs + (size_t)q * (kSlabBytes / 2));
       }
     }
   } else if (warp == kEpiThreads / 32) {
@@ -302,22 +295,20 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
           }
         }
         umma_commit(bar(B_L3));
-        if (train) {
-          // ---- dH2 = dZ3 W3 : acc1 = Z3[128 x 16] . slab[256 j x 16 o]^T
-          mbar_wait(bar(B_Z3), tpar);
+        // ---- dH2 = dZ3 W3 : acc1 = Z3[128 x 16] . slab[256 j x 16 o]^T
+        mbar_wait(bar(B_Z3), tpar);
+        tc_fence_after();
+        ring_mma(acc1, dZ3, 0u);
+        umma_commit(bar(B_D2));
+        // ---- dH1 = dZ2 W2 : acc0 = dZ2[128 x 256 j] . slab_s[256 i x 16 j]^T over the 16 j-steps
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          mbar_wait(bar(B_Z2C + j), tpar);
           tc_fence_after();
-          ring_mma(acc1, dZ3, 0u);
-          umma_commit(bar(B_D2));
-          // ---- dH1 = dZ2 W2 : acc0 = dZ2[128 x 256 j] . slab_s[256 i x 16 j]^T over the 16 j-steps
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            mbar_wait(bar(B_Z2C + j), tpar);
-            tc_fence_after();
-#pragma unroll
-            for (int h = 0; h < 4; ++h) ring_mma(acc0, dH2 + (uint64_t)(16 * (h * 4 + j)), (uint32_t)((j | h) != 0));
-          }
-          umma_commit(bar(B_D1));
+          for (int h = 0; h < 4; ++h) ring_mma(acc0, dH2 + (uint64_t)(16 * (h * 4 + j)), (uint32_t)((j | h) != 0));
         }
+        umma_commit(bar(B_D1));
         tpar ^= 1;
       }
     }
@@ -325,7 +316,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
     // ================================ staging + epilogue threads ==================================
     const int row = tid & (kRows - 1), grp = tid >> 7;
     const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
-    const int rps = (P.mode == MODE_CRITIC_TRAIN || (P.mode == MODE_FORWARD && C > 1)) ? 1 : P.M;   // rows per sample
+    const int rps = P.mode == MODE_CRITIC_TRAIN ? 1 : P.M;   // rows per sample
     const int n_pieces = K1p / 8;
     const bool vec4 = (D & 3) == 0;
     float4 xa[kMaxPieces], xb4[kMaxPieces];
@@ -386,7 +377,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
     };
     auto stage_x = [&](int xbuf, long long tile, int c) {
       bf16* dst = bufX + (size_t)xbuf * kRows * K1p;
-      bf16* gdst = train ? P.Xt + ((size_t)tile * C + c) * (size_t)kRows * K1p : nullptr;
+      bf16* gdst = P.Xt + ((size_t)tile * C + c) * (size_t)kRows * K1p;
 #pragma unroll
       for (int i = 0; i < kMaxPieces; ++i) {
         const int p = grp + i * 4;
@@ -395,7 +386,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
                                       pack_bf16(xb4[i].z, xb4[i].w));
           const size_t off = canon_off(row, p * 8, K1p);
           *reinterpret_cast<uint4*>(dst + off) = pk;
-          if (gdst != nullptr) *reinterpret_cast<uint4*>(gdst + off) = pk;
+          *reinterpret_cast<uint4*>(gdst + off) = pk;
         }
       }
     };
@@ -418,7 +409,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
           const uint4 pk = make_uint4(tanh2_bf16(z[0], z[1]), tanh2_bf16(z[2], z[3]), tanh2_bf16(z[4], z[5]), tanh2_bf16(z[6], z[7]));
           const size_t off = canon_off(row, c0 + q * 8, HID);
           *reinterpret_cast<uint4*>(sH + off) = pk;
-          if (gH != nullptr) *reinterpret_cast<uint4*>(gH + off) = pk;
+          *reinterpret_cast<uint4*>(gH + off) = pk;
         }
         proxy_fence();
         mbar_arrive(bar(chunk_bar + j));
@@ -485,7 +476,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
       // the row's loss inputs (a gather by sample index) are requested now and used two epilogues later: read at the
       // point of use they cost a DRAM latency on the tile's critical path (2 k of 35 k cycles in the phase trace)
       float pre_a[4] = {0.f, 0.f, 0.f, 0.f}, pre_lpo = 0.f, pre_adv = 0.f;
-      if (train && grp == 0 && samp >= 0) {
+      if (grp == 0 && samp >= 0) {
         if (P.mode == MODE_ACTOR_TRAIN) {
           const size_t arow = (size_t)samp * P.M + (int)((tile * kRows + row) % rps);
           for (int k = 0; k < W.out_dim; ++k) pre_a[k] = ldg_f1_pinned(P.act + arow * W.out_dim + k);
@@ -514,7 +505,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
       mbar_wait(bar(B_L1), tpar);
       tc_fence_after();
       if (tr) tr[2] = clock64();     // layer 1 complete
-      epi_forward(acc0, sB1, bufH1, train ? P.H1t + tbase : nullptr, B_H1C);
+      epi_forward(acc0, sB1, bufH1, P.H1t + tbase, B_H1C);
       tc_fence_before();
       if (tr) tr[3] = clock64();     // H1 written
       if (n2samp >= 0) {             // the row (actor) / the sample's M rows (critic) of the tile after the next one -> L2
@@ -528,7 +519,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
       mbar_wait(bar(B_L2), tpar);
       tc_fence_after();
       if (tr) tr[4] = clock64();     // layer 2 complete
-      epi_forward(acc1, sB2, bufH2, train ? P.H2t + tbase : nullptr, B_H2C);
+      epi_forward(acc1, sB2, bufH2, P.H2t + tbase, B_H2C);
       tc_fence_before();
       if (tr) tr[5] = clock64();     // H2 written
       // ---- output layer, loss, gradient at the output (column group 0 owns the rows)
@@ -539,14 +530,11 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
         uint32_t v[16];
         tmem_ld16_nowait(acc0 + lane_off, v);
         tmem_wait_ld();
-        const long long r = tile * kRows + row;
         float dz[4] = {0.f, 0.f, 0.f, 0.f};
         float loss = 0.f, kl = 0.f, dls[4] = {0.f, 0.f, 0.f, 0.f}, cntv = 0.f;
         if (samp >= 0) {
           cntv = 1.f;
-          if (P.mode == MODE_FORWARD) {
-            for (int k = 0; k < W.out_dim; ++k) P.out[(size_t)r * W.out_dim + k] = __uint_as_float(v[k]) + sB3[k];
-          } else if (P.mode == MODE_ACTOR_TRAIN) {
+          if (P.mode == MODE_ACTOR_TRAIN) {
             // agent.py:617-640 with torch.distributions.Normal.log_prob summed over the action dims
             float lp = 0.f, diff[4], ivar[4];
             for (int k = 0; k < W.out_dim; ++k) {
@@ -588,48 +576,44 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
             dz[0] = e;
           }
         }
-        if (train) {
-          // dZ3 tile [128 x 16] bf16, K-major (K = 16): my row's 16 entries = two core-matrix rows
-          const uint4 lo = make_uint4(pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u);
-          const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-          const size_t off = canon_off(row, 0, kNOut);
-          *reinterpret_cast<uint4*>(bufZ3 + off) = lo;
-          *reinterpret_cast<uint4*>(bufZ3 + off + 64) = zero;
-          bf16* g3 = P.dZ3t + (size_t)tile * kRows * kNOut;
-          *reinterpret_cast<uint4*>(g3 + off) = lo;
-          *reinterpret_cast<uint4*>(g3 + off + 64) = zero;
-          proxy_fence();
-          tc_fence_before();
-          mbar_arrive(bar(B_Z3));
-          if (tr) tr[13] = clock64();     // dZ3 handed to the tensor core
-          // tile statistics: warp reduce, then one shared-memory atomic per value and warp; the CTA's sums go to global
-          // memory once, when the kernel ends (11 double atomics per warp and tile on the same 11 addresses from every
-          // CTA cost ~4 k of a tile's 35 k cycles: profiles/r2_ppo_tile_trace_actor.txt)
-          float red[11] = {loss, kl, cntv, dls[0], dls[1], dls[2], dls[3], dz[0], dz[1], dz[2], dz[3]};
+        // dZ3 tile [128 x 16] bf16, K-major (K = 16): my row's 16 entries = two core-matrix rows
+        const uint4 lo = make_uint4(pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u);
+        const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+        const size_t off = canon_off(row, 0, kNOut);
+        *reinterpret_cast<uint4*>(bufZ3 + off) = lo;
+        *reinterpret_cast<uint4*>(bufZ3 + off + 64) = zero;
+        bf16* g3 = P.dZ3t + (size_t)tile * kRows * kNOut;
+        *reinterpret_cast<uint4*>(g3 + off) = lo;
+        *reinterpret_cast<uint4*>(g3 + off + 64) = zero;
+        proxy_fence();
+        tc_fence_before();
+        mbar_arrive(bar(B_Z3));
+        if (tr) tr[13] = clock64();     // dZ3 handed to the tensor core
+        // tile statistics: warp reduce, then one shared-memory atomic per value and warp; the CTA's sums go to global
+        // memory once, when the kernel ends (11 double atomics per warp and tile on the same 11 addresses from every
+        // CTA cost ~4 k of a tile's 35 k cycles: profiles/r2_ppo_tile_trace_actor.txt)
+        float red[11] = {loss, kl, cntv, dls[0], dls[1], dls[2], dls[3], dz[0], dz[1], dz[2], dz[3]};
 #pragma unroll
-          for (int i = 0; i < 11; ++i) {
-            float x = red[i];
-            for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-            if (lane == 0 && x != 0.f) atomicAdd(&s_red[i], x);
-          }
+        for (int i = 0; i < 11; ++i) {
+          float x = red[i];
+          for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+          if (lane == 0 && x != 0.f) atomicAdd(&s_red[i], x);
         }
       }
       if (tr) tr[7] = clock64();     // loss / output rows done
-      if (train) {
-        // ---- dZ2 = dH2 * (1 - H2^2), in place over H2; its chunks feed the dH1 MMAs
-        mbar_wait(bar(B_D2), tpar);
-        tc_fence_after();
-        if (tr) tr[8] = clock64();   // dH2 complete
-        epi_backward(acc1, bufH2, P.dZ2t + tbase, B_Z2C);
-        tc_fence_before();
-        if (tr) tr[9] = clock64();   // dZ2 written
-        // ---- dZ1 = dH1 * (1 - H1^2)
-        mbar_wait(bar(B_D1), tpar);
-        tc_fence_after();
-        if (tr) tr[10] = clock64();  // dH1 complete
-        epi_backward(acc0, bufH1, P.dZ1t + tbase, -1);
-        if (tr) tr[11] = clock64();  // dZ1 written
-      }
+      // ---- dZ2 = dH2 * (1 - H2^2), in place over H2; its chunks feed the dH1 MMAs
+      mbar_wait(bar(B_D2), tpar);
+      tc_fence_after();
+      if (tr) tr[8] = clock64();   // dH2 complete
+      epi_backward(acc1, bufH2, P.dZ2t + tbase, B_Z2C);
+      tc_fence_before();
+      if (tr) tr[9] = clock64();   // dZ2 written
+      // ---- dZ1 = dH1 * (1 - H1^2)
+      mbar_wait(bar(B_D1), tpar);
+      tc_fence_after();
+      if (tr) tr[10] = clock64();  // dH1 complete
+      epi_backward(acc0, bufH1, P.dZ1t + tbase, -1);
+      if (tr) tr[11] = clock64();  // dZ1 written
       tc_fence_before();
       mbar_arrive(bar(B_TDONE));
       tpar ^= 1;
@@ -637,7 +621,7 @@ mlp_tile_kernel(const __grid_constant__ TileArgs P) {
   }
   tc_fence_before();
   __syncthreads();
-  if (train && tid < 11 && s_red[tid] != 0.f) atomicAdd(P.stats + tid, (double)s_red[tid]);
+  if (tid < 11 && s_red[tid] != 0.f) atomicAdd(P.stats + tid, (double)s_red[tid]);
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u));
 }
 
@@ -1029,796 +1013,6 @@ int fwd2_stages(int K1p) {
   return st;
 }
 
-// ---------------------------------------------------------------------------------------------
-//          forward only on a CTA PAIR with resident weights (cta_group::2; actor nets, C == 1)
-// ---------------------------------------------------------------------------------------------
-// What bounds mlp_fwd2_kernel is the weight stream (a slab per ~340 cycles against the 128 an MMA needs).  A pair of CTAs
-// on the two SMs of a TPC executes M = 256 MMAs together: each CTA contributes its 128 rows of A and HALF of B (N / 2
-// rows of the weight matrix) from its own shared memory — so half of W1 / W2 / W3 (88 KB) fits next to two 64 KB
-// activation buffers and nothing is streamed.  Two cluster tiles (2 x 256 rows) are in flight, in alternation as in
-// mlp_fwd2_kernel; the inputs of a slot's next tile are staged into its activation buffer once its last layer has read
-// it.  Only the leader CTA's MMA thread issues; "operand ready" barriers live in the leader's shared memory and collect
-// the arrivals of BOTH CTAs' epilogue threads (remote arrive through mapa), "MMA done" commits are multicast to both.
-enum { C_W = 0, C_XFULL, C_L1 = C_XFULL + 2, C_L2 = C_L1 + 2, C_L3 = C_L2 + 2, C_H1 = C_L3 + 2, C_H2 = C_H1 + 2, C_COUNT = C_H2 + 2 };
-
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// arrive on the mbarrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_local, uint32_t rank) {
-  uint32_t remote;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(bar_local), "r"(rank));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_2cta(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_2cta(uint32_t mbar) {   // arrives on the barrier at this offset in BOTH CTAs
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(mbar),
-               "h"((uint16_t)3)
-               : "memory");
-}
-__host__ __device__ constexpr uint32_t umma_idesc_m256(int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-}
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
-mlp_fwd2c_kernel(const __grid_constant__ Fwd2Args P) {
-  extern __shared__ __align__(128) unsigned char smem_c2[];
-  const NetDev& W = P.net;
-  const int K1p = W.K1p, D = W.D;
-  bf16* const bufT0 = reinterpret_cast<bf16*>(smem_c2);                      // 2 x 64 KB: X -> H1 -> H2 per slot
-  bf16* const sW2 = bufT0 + 2 * (size_t)kRows * HID;                         // [128 n x 256] my half of W2
-  bf16* const sW1 = sW2 + (size_t)kRows * HID;                               // [128 n x K1p]
-  bf16* const sW3 = sW1 + (size_t)kRows * K1p;                               // [8 n x 256]
-  float* sB1 = reinterpret_cast<float*>(sW3 + (size_t)8 * HID);
-  float* sB2 = sB1 + HID;
-  float* sB3 = sB2 + HID;
-  float* sLs = sB3 + kNOut;
-  uint64_t* mbar = reinterpret_cast<uint64_t*>(sLs + kNOut);
-  uint32_t& tmem_base_s = *reinterpret_cast<uint32_t*>(mbar + C_COUNT);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  for (int i = tid; i < HID; i += kThreads) { sB1[i] = W.b1[i]; sB2[i] = W.b2[i]; }
-  if (tid < kNOut) { sB3[tid] = W.b3[tid]; sLs[tid] = W.logstd != nullptr ? W.logstd[tid] : 0.f; }
-  if (tid == 0) {
-    mbar_init(smem_u32(&mbar[C_W]), 1);
-    for (int i = 0; i < 2; ++i) {
-      // operand-ready barriers: used in the leader only, both CTAs' 512 epilogue threads arrive
-      mbar_init(smem_u32(&mbar[C_XFULL + i]), 2 * kEpiThreads);
-      mbar_init(smem_u32(&mbar[C_H1 + i]), 2 * kEpiThreads);
-      mbar_init(smem_u32(&mbar[C_H2 + i]), 2 * kEpiThreads);
-      // MMA-done barriers: one multicast commit each, in both CTAs
-      mbar_init(smem_u32(&mbar[C_L1 + i]), 1); mbar_init(smem_u32(&mbar[C_L2 + i]), 1); mbar_init(smem_u32(&mbar[C_L3 + i]), 1);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(512u));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::);
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();          // both CTAs' barriers exist before anybody arrives remotely
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_base_s;
-  const uint32_t bar0 = smem_u32(&mbar[0]);
-  auto bar = [&](int i) { return bar0 + 8u * (uint32_t)i; };
-  const uint32_t aT0 = smem_u32(bufT0), aW1 = smem_u32(sW1), aW2 = smem_u32(sW2), aW3 = smem_u32(sW3);
-  const uint32_t tbytes = (uint32_t)kRows * HID * 2u;
-  // cluster tiles of 256 rows: CTA `rank` owns rows [256 ct + 128 rank, + 128); cluster c takes ct = c, c + n_clusters, ...
-  const long long n_ct = (P.rows + 2 * kRows - 1) / (2 * kRows);
-  const long long cid = blockIdx.x >> 1, n_cl = gridDim.x >> 1;
-  const long long my_tiles = n_ct > cid ? (n_ct - cid + n_cl - 1) / n_cl : 0;
-  const int k1_steps = K1p / 16;
-
-  if (warp == kEpiThreads / 32) {
-    // ============================ weights (every CTA its half) + MMA issuer (leader) =============================
-    if (lane == 0) {
-      const uint32_t w1b = (uint32_t)(kRows * K1p * 2), w2b = (uint32_t)(kRows * HID * 2), w3b = (uint32_t)(8 * HID * 2);
-      mbar_expect_tx(bar(C_W), w1b + w2b + w3b);
-      bulk_g2s(aW1, W.w1c + (size_t)rank * kRows * K1p, w1b, bar(C_W));
-      bulk_g2s(aW2, W.w2c + (size_t)rank * kRows * HID, w2b, bar(C_W));
-      bulk_g2s(aW3, W.w3c + (size_t)rank * 8 * HID, w3b, bar(C_W));
-      mbar_wait(bar(C_W), 0);
-    }
-    __syncwarp();
-    // the leader may only issue once the PEER's weights have landed too
-    cluster_sync_all();
-    if (leader && lane == 0) {
-      const uint32_t sboX = (uint32_t)(K1p / 8) * 128u, sboH = (uint32_t)(HID / 8) * 128u;
-      const uint64_t dX = umma_desc(aT0, 128, sboX), dT = umma_desc(aT0, 128, sboH), dW1 = umma_desc(aW1, 128, sboX),
-                     dW2 = umma_desc(aW2, 128, sboH), dW3 = umma_desc(aW3, 128, sboH);
-      const uint64_t tstep = (uint64_t)(tbytes >> 4);
-      constexpr uint32_t kIdH = umma_idesc_m256(HID), kIdO = umma_idesc_m256(kNOut);
-      uint32_t ppar = 0;
-      for (long long p = 0; p < my_tiles; p += 2, ppar ^= 1) {
-        const int nt = (p + 1 < my_tiles) ? 2 : 1;
-#pragma unroll 1
-        for (int t = 0; t < nt; ++t) {                     // layer 1
-          const uint32_t acc = tmem_base + (uint32_t)t * HID;
-          mbar_wait_cluster(bar(C_XFULL + t), ppar);
-          tc_fence_after();
-          const uint64_t a = dX + tstep * (uint64_t)t;
-          for (int s = 0; s < k1_steps; ++s) umma_bf16_2cta(acc, a + (uint64_t)(16 * s), dW1 + (uint64_t)(16 * s), kIdH, (uint32_t)(s != 0));
-          umma_commit_2cta(bar(C_L1 + t));
-        }
-#pragma unroll 1
-        for (int t = 0; t < nt; ++t) {                     // layer 2
-          const uint32_t acc = tmem_base + (uint32_t)t * HID;
-          mbar_wait_cluster(bar(C_H1 + t), ppar);
-          tc_fence_after();
-          const uint64_t a = dT + tstep * (uint64_t)t;
-#pragma unroll
-          for (int s = 0; s < 16; ++s) umma_bf16_2cta(acc, a + (uint64_t)(16 * s), dW2 + (uint64_t)(16 * s), kIdH, (uint32_t)(s != 0));
-          umma_commit_2cta(bar(C_L2 + t));
-        }
-#pragma unroll 1
-        for (int t = 0; t < nt; ++t) {                     // layer 3, N = 16
-          const uint32_t acc = tmem_base + (uint32_t)t * HID;
-          mbar_wait_cluster(bar(C_H2 + t), ppar);
-          tc_fence_after();
-          const uint64_t a = dT + tstep * (uint64_t)t;
-#pragma unroll
-          for (int s = 0; s < 16; ++s) umma_bf16_2cta(acc, a + (uint64_t)(16 * s), dW3 + (uint64_t)(16 * s), kIdO, (uint32_t)(s != 0));
-          umma_commit_2cta(bar(C_L3 + t));
-        }
-      }
-    }
-  } else if (warp < kEpiThreads / 32) {
-    // ================================ staging + epilogue threads ==================================
-    const int row = tid & (kRows - 1), grp = tid >> 7;
-    const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
-    const int rps = P.rows_per_sample;
-    const int n_pieces = K1p / 8;
-    const bool vec4 = (D & 3) == 0;
-    float4 xa[kMaxPieces], xb4[kMaxPieces];
-    cluster_sync_all();          // matches the MMA warp's second cluster barrier (weights landed everywhere)
-
-    auto ctile_of = [&](long long pos) { return cid + pos * n_cl; };
-    auto row_of = [&](long long ct) { return ct * (2 * kRows) + (long long)rank * kRows + row; };
-    auto sample_of = [&](long long ct) -> long long {
-      const long long r = row_of(ct);
-      if (r >= P.rows) return -1;
-      const long long smp = r / rps;
-      return P.idx != nullptr ? P.idx[smp] : smp;
-    };
-    auto load_x = [&](long long ct, long long sm) {
-      const long long r = row_of(ct);
-      const int agent = (int)(r % rps);
-      const float* src = P.obs + ((size_t)(sm < 0 ? 0 : sm) * P.M + agent) * D;
-#pragma unroll
-      for (int i = 0; i < kMaxPieces; ++i) {
-        const int k0 = (grp + i * 4) * 8;
-        xa[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        xb4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (k0 < D && sm >= 0) {
-          if (vec4 && k0 + 8 <= D) {
-            xa[i] = __ldg(reinterpret_cast<const float4*>(src + k0));
-            xb4[i] = __ldg(reinterpret_cast<const float4*>(src + k0 + 4));
-          } else {
-            float x[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) x[j] = (k0 + j < D) ? __ldg(src + k0 + j) : 0.0f;
-            xa[i] = make_float4(x[0], x[1], x[2], x[3]);
-            xb4[i] = make_float4(x[4], x[5], x[6], x[7]);
-          }
-        }
-      }
-    };
-    // registers -> (normalise) -> bf16 canonical [128 x K1p] at the start of slot t's activation buffer
-    auto stage_x = [&](int t, long long ct, long long sm) {
-      const long long r = row_of(ct);
-      const int agent = (int)(r % rps);
-      bf16* dst = bufT0 + (size_t)t * kRows * HID;
-      const bool norm = P.nmean != nullptr && sm >= 0;
-      const size_t nb = norm ? ((size_t)(sm / P.N) * P.M + agent) * D : 0;
-#pragma unroll
-      for (int i = 0; i < kMaxPieces; ++i) {
-        const int pc = grp + i * 4;
-        if (pc < n_pieces) {
-          float x[8] = {xa[i].x, xa[i].y, xa[i].z, xa[i].w, xb4[i].x, xb4[i].y, xb4[i].z, xb4[i].w};
-          if (norm) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const int k = pc * 8 + j;
-              if (k < D) {
-                const float v = (x[j] - __ldg(P.nmean + nb + k)) * __ldg(P.nrstd + nb + k);
-                x[j] = fminf(fmaxf(v, -P.nclip), P.nclip);
-              }
-            }
-          }
-          *reinterpret_cast<uint4*>(dst + canon_off(row, pc * 8, K1p)) =
-              make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
-        }
-      }
-      proxy_fence();
-      tc_fence_before();
-      mbar_arrive_cluster(bar(C_XFULL + t), 0);
-    };
-    auto epi_hidden = [&](uint32_t acc, const float* bias, bf16* sH, int done_bar) {
-      uint32_t va[16], vb[16];
-      tmem_ld16_nowait(acc + lane_off + (uint32_t)(grp * 64), va);
-      tmem_wait_ld();
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int c0 = grp * 64 + j * 16;
-        uint32_t* cur = (j & 1) ? vb : va;
-        uint32_t* nxt = (j & 1) ? va : vb;
-        if (j < 3) tmem_ld16_nowait(acc + lane_off + (uint32_t)(c0 + 16), nxt);
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          float z[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) z[e] = __uint_as_float(cur[q * 8 + e]) + bias[c0 + q * 8 + e];
-          *reinterpret_cast<uint4*>(sH + canon_off(row, c0 + q * 8, HID)) =
-              make_uint4(tanh2_bf16(z[0], z[1]), tanh2_bf16(z[2], z[3]), tanh2_bf16(z[4], z[5]), tanh2_bf16(z[6], z[7]));
-        }
-        tmem_wait_ld();
-      }
-      proxy_fence();
-      tc_fence_before();
-      mbar_arrive_cluster(bar(done_bar), 0);
-    };
-    auto finish_row = [&](long long r, const uint32_t (&v)[16]) {
-      if (!P.sample) {
-        for (int k = 0; k < W.out_dim; ++k) P.out[(size_t)r * W.out_dim + k] = __uint_as_float(v[k]) + sB3[k];
-        return;
-      }
-      float eps[4] = {0.f, 0.f, 0.f, 0.f};
-      if (P.noise != nullptr) {
-        for (int k = 0; k < W.out_dim; ++k) eps[k] = P.noise[(size_t)r * W.out_dim + k];
-      } else {
-        uint32_t c[4] = {(uint32_t)r, (uint32_t)((unsigned long long)r >> 32), (uint32_t)P.offset, (uint32_t)(P.offset >> 32)};
-        philox4x32_10(c, (uint32_t)P.seed, (uint32_t)(P.seed >> 32));
-        const float u0 = ((c[0] >> 8) + 0.5f) * (1.0f / 16777216.0f), u1 = (c[1] >> 8) * (1.0f / 16777216.0f);
-        const float u2 = ((c[2] >> 8) + 0.5f) * (1.0f / 16777216.0f), u3 = (c[3] >> 8) * (1.0f / 16777216.0f);
-        const float r0 = sqrtf(-2.0f * __logf(u0)), r1 = sqrtf(-2.0f * __logf(u2));
-        float s0, c0, s1, c1;
-        __sincosf(6.28318530718f * u1, &s0, &c0);
-        __sincosf(6.28318530718f * u3, &s1, &c1);
-        eps[0] = r0 * c0; eps[1] = r0 * s0; eps[2] = r1 * c1; eps[3] = r1 * s1;
-      }
-      float lp = 0.f;
-      for (int k = 0; k < W.out_dim; ++k) {
-        const float m = __uint_as_float(v[k]) + sB3[k];
-        const float ls = sLs[k];
-        P.out[(size_t)r * W.out_dim + k] = fmaf(__expf(ls), eps[k], m);
-        if (P.mean_out != nullptr) P.mean_out[(size_t)r * W.out_dim + k] = m;
-        lp += -0.5f * eps[k] * eps[k] - ls - 0.91893853320467f;
-      }
-      P.logp[r] = lp;
-    };
-
-    // prologue: both slots' first tiles
-#pragma unroll 1
-    for (int t = 0; t < 2; ++t)
-      if (t < my_tiles) {
-        const long long ct = ctile_of(t), sm = sample_of(ct);
-        load_x(ct, sm);
-        stage_x(t, ct, sm);
-      }
-    uint32_t ppar = 0;
-    long long* const tr0 = (P.trace != nullptr && blockIdx.x == 0 && tid == 0) ? P.trace : nullptr;
-    for (long long p = 0; p < my_tiles; p += 2, ppar ^= 1) {
-      const int nt = (p + 1 < my_tiles) ? 2 : 1;
-      long long* const tr = (tr0 != nullptr && p < 64) ? tr0 + (p >> 1) * 64 : nullptr;
-      if (tr) tr[0] = clock64();
-#pragma unroll 1
-      for (int lt = 0; lt < 4; ++lt) {                     // H1(A), H1(B), H2(A), H2(B)
-        const int layer = lt >> 1, t = lt & 1;
-        if (t >= nt) continue;
-        mbar_wait(bar(C_L1 + 2 * layer + t), ppar);
-        tc_fence_after();
-        if (tr) tr[1 + 2 * lt] = clock64();                // accumulator ready
-        epi_hidden(tmem_base + (uint32_t)t * HID, layer ? sB2 : sB1, bufT0 + (size_t)t * kRows * HID, C_H1 + 2 * layer + t);
-        if (tr) tr[2 + 2 * lt] = clock64();                // epilogue done
-      }
-#pragma unroll 1
-      for (int t = 0; t < nt; ++t) {                       // outputs; then the slot's next inputs into its (now free) buffer
-        const bool has_next = p + t + 2 < my_tiles;
-        const long long nct = ctile_of(p + t + 2);
-        long long nsm = -1;
-        if (has_next) { nsm = sample_of(nct); load_x(nct, nsm); }
-        mbar_wait(bar(C_L3 + t), ppar);
-        tc_fence_after();
-        if (tr) tr[9 + 3 * t] = clock64();                 // output accumulator ready
-        uint32_t v[16];
-        if (grp == 0) { tmem_ld16_nowait(tmem_base + (uint32_t)t * HID + lane_off, v); tmem_wait_ld(); }
-        if (has_next) stage_x(t, nct, nsm);               // (arrives after my read of the accumulator)
-        if (tr) tr[10 + 3 * t] = clock64();                // next inputs staged
-        const long long r = row_of(ctile_of(p + t));
-        if (grp == 0 && r < P.rows) finish_row(r, v);
-        if (tr) tr[11 + 3 * t] = clock64();                // rows written
-      }
-    }
-  } else {
-    cluster_sync_all();          // the spare warp only takes part in the cluster barriers
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();            // nobody leaves (and frees tensor memory the pair shares) before the peer is done
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u));
-}
-size_t fwd2c_kernel_smem(int K1p) {
-  return (size_t)2 * kRows * HID * 2 + (size_t)kRows * HID * 2 + (size_t)kRows * K1p * 2 + (size_t)8 * HID * 2 +
-         (size_t)(2 * HID + 2 * kNOut) * 4 + (size_t)C_COUNT * 8 + 16;
-}
-
-// ---------------------------------------------------------------------------------------------
-//              forward + loss + backward with TWO tiles in flight per CTA (training, round 2)
-// ---------------------------------------------------------------------------------------------
-// mlp_tile_kernel takes one tile at a time through ten dependent phases (MMA, epilogue, MMA, ...): 34 k cycles per tile
-// of which the tensor pipe works 12 % (profiles/r2_ppo_tile_trace_actor.txt).  Two observations make a second tile fit:
-//   * H1 is an MMA operand only for layer 2; the backward pass needs it element-wise (dZ1 = dH1 (1 - H1^2)), and the
-//     thread that needs an element is the thread that wrote it to the H1 tile in global memory (for the weight-gradient
-//     kernel) — so H2 can overwrite H1 in shared memory (after layer 2 has completed) and H1 is re-read from global;
-//   * dZ1 is never an MMA operand here (only in dw_kernel): it goes to global memory and nowhere else.
-// A tile therefore needs ONE 64 KB activation buffer (H1 -> H2 -> dZ2, all in place), its input buffer and a 4 KB dZ3
-// tile, and one 256-column accumulator when the next MMA phase starts only after the previous epilogue has finished —
-// which costs nothing once a second tile keeps both units busy: the tensor core runs phase k of tile B while the 512
-// epilogue threads finish phase k of tile A.  Same roles, ring and barrier style as mlp_fwd2_kernel.
-// Phases per slot t:  L1 -> H1 | L2 -> H2 | L3 -> loss (-> dZ3) | D2 (dH2) -> dZ2 | D1 (dH1) -> dZ1.
-enum { T_W3 = 0, T_XFULL, T_XEMPTY = T_XFULL + 2, T_L1 = T_XEMPTY + 2, T_L2 = T_L1 + 2, T_L3 = T_L2 + 2, T_D2 = T_L3 + 2,
-       T_D1 = T_D2 + 2, T_H1 = T_D1 + 2, T_H2 = T_H1 + 2, T_Z3 = T_H2 + 2, T_Z2 = T_Z3 + 2, T_OUT = T_Z2 + 2, T_FULL = T_OUT + 2,
-       T_EMPTY = T_FULL + kMaxStages, T_COUNT = T_EMPTY + kMaxStages };
-
-__global__ void __launch_bounds__(kThreads, 1)
-mlp_train2_kernel(const __grid_constant__ TileArgs P) {
-  extern __shared__ __align__(128) unsigned char smem_t2[];
-  const NetDev& W = P.net;
-  const int K1p = W.K1p, C = W.C, D = W.D, stages = P.stages;
-  bf16* const bufT0 = reinterpret_cast<bf16*>(smem_t2);                      // 2 x 64 KB: H1 -> H2 -> dZ2
-  bf16* const bufX0 = bufT0 + 2 * (size_t)kRows * HID;                       // 2 x [128 x K1p]
-  const uint32_t xbytes = (uint32_t)kRows * (uint32_t)K1p * 2u;
-  bf16* const bufZ0 = bufX0 + 2 * (size_t)kRows * K1p;                       // 2 x [128 x 16]
-  bf16* sW3 = bufZ0 + 2 * (size_t)kRows * kNOut;
-  unsigned char* ring = reinterpret_cast<unsigned char*>(sW3 + (size_t)kNOut * HID);
-  float* sB1 = reinterpret_cast<float*>(ring + (size_t)stages * kSlabBytes);
-  float* sB2 = sB1 + HID;
-  float* sB3 = sB2 + HID;
-  float* sLs = sB3 + kNOut;
-  float* s_red = sLs + kNOut;                                                // [16] CTA-wide statistics
-  uint64_t* mbar = reinterpret_cast<uint64_t*>(s_red + 16);
-  uint32_t& tmem_base_s = *reinterpret_cast<uint32_t*>(mbar + T_COUNT);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  for (int i = tid; i < HID; i += kThreads) { sB1[i] = W.b1[i]; sB2[i] = W.b2[i]; }
-  if (tid < kNOut) { sB3[tid] = W.b3[tid]; sLs[tid] = W.logstd != nullptr ? W.logstd[tid] : 0.f; s_red[tid] = 0.f; }
-  if (tid == 0) {
-    mbar_init(smem_u32(&mbar[T_W3]), 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(smem_u32(&mbar[T_XFULL + i]), kEpiThreads); mbar_init(smem_u32(&mbar[T_XEMPTY + i]), 1);
-      mbar_init(smem_u32(&mbar[T_L1 + i]), 1); mbar_init(smem_u32(&mbar[T_L2 + i]), 1); mbar_init(smem_u32(&mbar[T_L3 + i]), 1);
-      mbar_init(smem_u32(&mbar[T_D2 + i]), 1); mbar_init(smem_u32(&mbar[T_D1 + i]), 1);
-      mbar_init(smem_u32(&mbar[T_H1 + i]), kEpiThreads); mbar_init(smem_u32(&mbar[T_H2 + i]), kEpiThreads);
-      mbar_init(smem_u32(&mbar[T_Z3 + i]), kRows); mbar_init(smem_u32(&mbar[T_Z2 + i]), kEpiThreads);
-      mbar_init(smem_u32(&mbar[T_OUT + i]), kEpiThreads);
-    }
-    for (int i = 0; i < kMaxStages; ++i) { mbar_init(smem_u32(&mbar[T_FULL + i]), 1); mbar_init(smem_u32(&mbar[T_EMPTY + i]), 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_s)), "r"(512u));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_base_s;
-  const uint32_t bar0 = smem_u32(&mbar[0]);
-  auto bar = [&](int i) { return bar0 + 8u * (uint32_t)i; };
-  const uint32_t aT0 = smem_u32(bufT0), aX0 = smem_u32(bufX0), aZ0 = smem_u32(bufZ0), aW3 = smem_u32(sW3), aRing = smem_u32(ring);
-  const uint32_t tbytes = (uint32_t)kRows * HID * 2u, zbytes = (uint32_t)kRows * kNOut * 2u;
-  const long long n_tiles = (P.rows + kRows - 1) / kRows;
-  const long long my_tiles = n_tiles > (long long)blockIdx.x ? (n_tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-  const int k1_steps = K1p / 16;
-
-  if (warp == kEpiThreads / 32 + 1) {
-    // ===================================== TMA producer ===========================================
-    if (lane == 0) {
-      mbar_expect_tx(bar(T_W3), (uint32_t)(kNOut * HID * 2));
-      bulk_g2s(aW3, W.w3f, (uint32_t)(kNOut * HID * 2), bar(T_W3));
-      uint32_t st = 0, epar = 1, lap0 = 1;
-      const uint64_t keep = l2_policy_evict_last();
-      auto push = [&](const bf16* src) {
-        if (!lap0) mbar_wait(bar(T_EMPTY + (int)st), epar);
-        mbar_expect_tx(bar(T_FULL + (int)st), kSlabBytes);
-        bulk_g2s_hint(aRing + st * kSlabBytes, src, kSlabBytes, bar(T_FULL + (int)st), keep);
-        if (++st == (uint32_t)stages) { st = 0; epar ^= 1; lap0 = 0; }
-      };
-      const int n1 = C * k1_steps;
-      for (long long p = 0; p < my_tiles; p += 2) {            // ONE set of slabs per pair: every slab serves both tiles
-        for (int q = 0; q < n1; ++q) push(W.w1_slabs + (size_t)q * (kSlabBytes / 2));
-        for (int q = 0; q < 16; ++q) push(W.w2f_slabs + (size_t)q * (kSlabBytes / 2));
-        push(W.w3b_slab);
-        for (int q = 0; q < 16; ++q) push(W.w2b_slabs + (size_t)q * (kSlabBytes / 2));
-      }
-    }
-  } else if (warp == kEpiThreads / 32) {
-    // ===================================== MMA issuer =============================================
-    if (lane == 0) {
-      uint32_t st = 0, fpar = 0;
-      uint32_t xpar = 0;                 // bit t: parity of slot t's next XFULL completion
-      const uint32_t sboX = (uint32_t)(K1p / 8) * 128u, sboH = (uint32_t)(HID / 8) * 128u;
-      const uint64_t dX = umma_desc(aX0, 128, sboX), dT = umma_desc(aT0, 128, sboH), dW3 = umma_desc(aW3, 128, sboH),
-                     dZ = umma_desc(aZ0, 128, 256), dRing = umma_desc(aRing, 128, 256);
-      const uint64_t xstep = (uint64_t)(xbytes >> 4), tstep = (uint64_t)(tbytes >> 4), zstep = (uint64_t)(zbytes >> 4);
-      constexpr uint32_t kIdH = umma_idesc(HID), kIdO = umma_idesc(kNOut);
-      // one streamed K-step for BOTH slots: wait for the slab, issue one MMA per tile of the pair on it, hand the stage
-      // back.  The slab stream is what bounds this kernel (an 8 KB slab arrives every 300-800 cycles with the 5 stages
-      // that fit, profiles/r2_ppo_train2_trace.txt), so a fetch has to feed as many rows as possible.
-      auto ring_mma2 = [&](int nt, uint64_t adescA, uint64_t adescB, uint32_t accumulate) {
-        mbar_wait(bar(T_FULL + (int)st), fpar);
-        const uint64_t b = dRing + (uint64_t)(st * (kSlabBytes >> 4));
-        umma_bf16(tmem_base, adescA, b, kIdH, accumulate);
-        if (nt > 1) umma_bf16(tmem_base + (uint32_t)HID, adescB, b, kIdH, accumulate);
-        umma_commit(bar(T_EMPTY + (int)st));
-        if (++st == (uint32_t)stages) { st = 0; fpar ^= 1; }
-      };
-      mbar_wait(bar(T_W3), 0);
-      uint32_t ppar = 0;
-      for (long long p = 0; p < my_tiles; p += 2, ppar ^= 1) {
-        const int nt = (p + 1 < my_tiles) ? 2 : 1;
-        // ---- layer 1 of both tiles
-        if (p > 0)
-          for (int t = 0; t < nt; ++t) { mbar_wait(bar(T_OUT + t), ppar ^ 1); }   // the slots' previous tiles are through
-        tc_fence_after();
-#pragma unroll 1
-        for (int c = 0; c < C; ++c) {
-          for (int t = 0; t < nt; ++t) { mbar_wait(bar(T_XFULL + t), (xpar >> t) & 1u); xpar ^= 1u << t; }
-          tc_fence_after();
-          for (int s = 0; s < k1_steps; ++s) ring_mma2(nt, dX + (uint64_t)(16 * s), dX + xstep + (uint64_t)(16 * s), (uint32_t)((c | s) != 0));
-          for (int t = 0; t < nt; ++t) umma_commit(bar(T_XEMPTY + t));
-        }
-        for (int t = 0; t < nt; ++t) umma_commit(bar(T_L1 + t));
-        // ---- layer 2: H1 W2^T
-        for (int t = 0; t < nt; ++t) mbar_wait(bar(T_H1 + t), ppar);
-        tc_fence_after();
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          const uint64_t o = (uint64_t)(16 * (4 * (i & 3) + (i >> 2)));
-          ring_mma2(nt, dT + o, dT + tstep + o, (uint32_t)(i != 0));
-        }
-        for (int t = 0; t < nt; ++t) umma_commit(bar(T_L2 + t));
-        // ---- layer 3: H2 W3^T (resident), N = 16, per slot as its H2 arrives
-#pragma unroll 1
-        for (int t = 0; t < nt; ++t) {
-          const uint32_t acc = tmem_base + (uint32_t)t * HID;
-          mbar_wait(bar(T_H2 + t), ppar);
-          tc_fence_after();
-          const uint64_t dTt = dT + tstep * (uint64_t)t;
-#pragma unroll
-          for (int s = 0; s < 16; ++s) umma_bf16(acc, dTt + (uint64_t)(16 * s), dW3 + (uint64_t)(16 * s), kIdO, (uint32_t)(s != 0));
-          umma_commit(bar(T_L3 + t));
-        }
-        // ---- dH2 = dZ3 W3: one K = 16 step over the W3^T slab
-        for (int t = 0; t < nt; ++t) mbar_wait(bar(T_Z3 + t), ppar);
-        tc_fence_after();
-        ring_mma2(nt, dZ, dZ + zstep, 0u);
-        for (int t = 0; t < nt; ++t) umma_commit(bar(T_D2 + t));
-        // ---- dH1 = dZ2 W2 over the 16 W2^T slabs
-        for (int t = 0; t < nt; ++t) mbar_wait(bar(T_Z2 + t), ppar);
-        tc_fence_after();
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          const uint64_t o = (uint64_t)(16 * (4 * (i & 3) + (i >> 2)));
-          ring_mma2(nt, dT + o, dT + tstep + o, (uint32_t)(i != 0));
-        }
-        for (int t = 0; t < nt; ++t) umma_commit(bar(T_D1 + t));
-      }
-    }
-  } else {
-    // ================================ staging + epilogue threads ==================================
-    const int row = tid & (kRows - 1), grp = tid >> 7;
-    const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
-    const int rps = (P.mode == MODE_CRITIC_TRAIN) ? 1 : P.M;
-    const int n_pieces = K1p / 8;
-    const bool vec4 = (D & 3) == 0;
-    float4 xa[kMaxPieces], xb4[kMaxPieces];
-    uint32_t xe = 0, xused = 0;
-
-    auto tile_of = [&](long long pos) { return (long long)blockIdx.x + pos * gridDim.x; };
-    auto sample_of = [&](long long tile) -> long long {
-      const long long r = tile * kRows + row;
-      if (r >= P.rows) return -1;
-      const long long s = r / rps;
-      return P.idx != nullptr ? P.idx[s] : s;
-    };
-    auto load_x = [&](long long tile, int c, long long sm) {
-      const long long r = tile * kRows + row;
-      const int agent = (rps == 1) ? c : (int)(r % rps);
-      const float* src = P.obs + ((size_t)(sm < 0 ? 0 : sm) * P.M + agent) * D;
-#pragma unroll
-      for (int i = 0; i < kMaxPieces; ++i) {
-        const int k0 = (grp + i * 4) * 8;
-        xa[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        xb4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (k0 < D && sm >= 0) {
-          if (vec4 && k0 + 8 <= D) {
-            xa[i] = __ldg(reinterpret_cast<const float4*>(src + k0));
-            xb4[i] = __ldg(reinterpret_cast<const float4*>(src + k0 + 4));
-          } else {
-            float x[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) x[j] = (k0 + j < D) ? __ldg(src + k0 + j) : 0.0f;
-            xa[i] = make_float4(x[0], x[1], x[2], x[3]);
-            xb4[i] = make_float4(x[4], x[5], x[6], x[7]);
-          }
-        }
-      }
-    };
-    // registers -> (normalise) -> bf16 canonical tile of slot t (+ the global copy dw_kernel reads)
-    auto stage_x = [&](int t, long long tile, int c, long long sm) {
-      const long long r = tile * kRows + row;
-      const int agent = (rps == 1) ? c : (int)(r % rps);
-      if ((xused >> t) & 1u) { mbar_wait(bar(T_XEMPTY + t), (xe >> t) & 1u); xe ^= 1u << t; }
-      xused |= 1u << t;
-      bf16* dst = reinterpret_cast<bf16*>(reinterpret_cast<unsigned char*>(bufX0) + (size_t)t * xbytes);
-      bf16* gdst = P.Xt + ((size_t)tile * C + c) * (size_t)kRows * K1p;
-      const bool norm = P.nmean != nullptr && sm >= 0;
-      const size_t nb = norm ? ((size_t)(sm / P.N) * P.M + agent) * D : 0;
-#pragma unroll
-      for (int i = 0; i < kMaxPieces; ++i) {
-        const int pc = grp + i * 4;
-        if (pc < n_pieces) {
-          float x[8] = {xa[i].x, xa[i].y, xa[i].z, xa[i].w, xb4[i].x, xb4[i].y, xb4[i].z, xb4[i].w};
-          if (norm) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const int k = pc * 8 + j;
-              if (k < D) {
-                const float v = (x[j] - __ldg(P.nmean + nb + k)) * __ldg(P.nrstd + nb + k);
-                x[j] = fminf(fmaxf(v, -P.nclip), P.nclip);
-              }
-            }
-          }
-          const uint4 pk = make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
-          const size_t off = canon_off(row, pc * 8, K1p);
-          *reinterpret_cast<uint4*>(dst + off) = pk;
-          __stcs(reinterpret_cast<uint4*>(gdst + off), pk);
-        }
-      }
-      proxy_fence();
-      mbar_arrive(bar(T_XFULL + t));
-    };
-    // forward epilogue: acc row -> +bias, tanh -> bf16 -> the slot's activation tile and its global copy
-    auto epi_forward = [&](uint32_t acc, const float* bias, bf16* sH, bf16* gH, int done_bar) {
-      uint32_t va[16], vb[16];
-      tmem_ld16_nowait(acc + lane_off + (uint32_t)(grp * 64), va);
-      tmem_wait_ld();
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int c0 = grp * 64 + j * 16;
-        uint32_t* cur = (j & 1) ? vb : va;
-        uint32_t* nxt = (j & 1) ? va : vb;
-        if (j < 3) tmem_ld16_nowait(acc + lane_off + (uint32_t)(c0 + 16), nxt);
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          float z[8];
-#pragma unroll
-          for (int e = 0; e < 8; ++e) z[e] = __uint_as_float(cur[q * 8 + e]) + bias[c0 + q * 8 + e];
-          const uint4 pk = make_uint4(tanh2_bf16(z[0], z[1]), tanh2_bf16(z[2], z[3]), tanh2_bf16(z[4], z[5]), tanh2_bf16(z[6], z[7]));
-          const size_t off = canon_off(row, c0 + q * 8, HID);
-          *reinterpret_cast<uint4*>(sH + off) = pk;
-          __stcs(reinterpret_cast<uint4*>(gH + off), pk);
-        }
-        tmem_wait_ld();
-      }
-      proxy_fence();
-      tc_fence_before();
-      mbar_arrive(bar(done_bar));
-    };
-    // backward epilogue: dZ = dH (1 - H^2) with H from `hsrc` (shared: H2, in place; global: my own H1 copy);
-    // dZ -> `sdst` (shared, may be null) and the global tile `gZ`
-    auto epi_backward = [&](uint32_t acc, const bf16* hsrc, bf16* sdst, bf16* gZ, int done_bar) {
-      uint32_t va[16], vb[16];
-      tmem_ld16_nowait(acc + lane_off + (uint32_t)(grp * 64), va);
-      tmem_wait_ld();
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int c0 = grp * 64 + j * 16;
-        uint32_t* cur = (j & 1) ? vb : va;
-        uint32_t* nxt = (j & 1) ? va : vb;
-        if (j < 3) tmem_ld16_nowait(acc + lane_off + (uint32_t)(c0 + 16), nxt);
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-          const size_t off = canon_off(row, c0 + q * 8, HID);
-          const uint4 hv = *reinterpret_cast<const uint4*>(hsrc + off);
-          const uint32_t hw[4] = {hv.x, hv.y, hv.z, hv.w};
-          uint32_t o[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            float h0, h1;
-            unpack_bf16(hw[e], h0, h1);
-            const float d0 = __uint_as_float(cur[q * 8 + 2 * e]) * fmaf(-h0, h0, 1.0f);
-            const float d1 = __uint_as_float(cur[q * 8 + 2 * e + 1]) * fmaf(-h1, h1, 1.0f);
-            o[e] = pack_bf16(d0, d1);
-          }
-          const uint4 pk = make_uint4(o[0], o[1], o[2], o[3]);
-          if (sdst != nullptr) *reinterpret_cast<uint4*>(sdst + off) = pk;
-          __stcs(reinterpret_cast<uint4*>(gZ + off), pk);
-        }
-        tmem_wait_ld();
-      }
-      if (sdst != nullptr) proxy_fence();
-      tc_fence_before();
-      mbar_arrive(bar(done_bar));
-    };
-
-    // prologue: chunk 0 of both slots' first tiles
-#pragma unroll 1
-    for (int t = 0; t < 2; ++t)
-      if (t < my_tiles) {
-        const long long tile = tile_of(t), sm = sample_of(tile);
-        load_x(tile, 0, sm);
-        stage_x(t, tile, 0, sm);
-      }
-    uint32_t ppar = 0;
-    long long* const tr0 = (P.trace != nullptr && blockIdx.x == 0 && tid == 0) ? P.trace : nullptr;
-    for (long long p = 0; p < my_tiles; p += 2, ppar ^= 1) {
-      const int nt = (p + 1 < my_tiles) ? 2 : 1;
-      long long* const tr = (tr0 != nullptr && p < 32) ? tr0 + (p >> 1) * 16 : nullptr;   // [pair][16] stamps of thread 0
-      if (tr) tr[0] = clock64();
-      if (C > 1) {     // centralised critic: the remaining input chunks of the current tiles, one by one
-        // (chunk by chunk over BOTH slots: the tensor core consumes chunk c of the two tiles together)
-#pragma unroll 1
-        for (int c = 1; c < C; ++c)
-#pragma unroll 1
-          for (int t = 0; t < nt; ++t) {
-            const long long tile = tile_of(p + t), sm = sample_of(tile);
-            load_x(tile, c, sm);
-            stage_x(t, tile, c, sm);
-          }
-      }
-      // ---- hidden layers: H1 of A while the tensor core runs layer 1 of B, H1 of B during layer 2 of A, ...
-#pragma unroll 1
-      for (int lt = 0; lt < 4; ++lt) {
-        const int layer = lt >> 1, t = lt & 1;
-        if (t >= nt) continue;
-        const long long tile = tile_of(p + t);
-        const bool has_next = layer == 0 && p + t + 2 < my_tiles;
-        const long long ntile = tile_of(p + t + 2);
-        long long nsm = -1;
-        if (has_next) { nsm = sample_of(ntile); load_x(ntile, 0, nsm); }   // in flight during the epilogue below
-        mbar_wait(bar(T_L1 + 2 * layer + t), ppar);
-        tc_fence_after();
-        epi_forward(tmem_base + (uint32_t)t * HID, layer ? sB2 : sB1, bufT0 + (size_t)t * kRows * HID,
-                    (layer ? P.H2t : P.H1t) + (size_t)tile * kRows * HID, T_H1 + 2 * layer + t);
-        if (has_next) stage_x(t, ntile, 0, nsm);           // layer 1 of this tile is complete: its input buffer is free
-        if (tr) tr[1 + lt] = clock64();                    // H1(A), H1(B), H2(A), H2(B) done
-      }
-      // ---- output layer, loss, gradient at the output (column group 0 owns the rows)
-      if (grp == 0) {
-#pragma unroll 1
-        for (int t = 0; t < nt; ++t) {
-          const long long tile = tile_of(p + t);
-          const long long r = tile * kRows + row;
-          const long long samp = sample_of(tile);
-          float pre_a[4] = {0.f, 0.f, 0.f, 0.f}, pre_lpo = 0.f, pre_adv = 0.f;
-          if (samp >= 0) {                                 // requested before the wait for layer 3
-            if (P.mode == MODE_ACTOR_TRAIN) {
-              const size_t arow = (size_t)samp * P.M + (int)(r % rps);
-              for (int k = 0; k < W.out_dim; ++k) pre_a[k] = __ldg(P.act + arow * W.out_dim + k);
-              pre_lpo = __ldg(P.logp_old + arow);
-              pre_adv = __ldg(P.adv + samp);
-            } else {
-              pre_adv = __ldg(P.ret + samp);
-              if (P.use_clipped_value > 0.f && P.v_old != nullptr) pre_lpo = __ldg(P.v_old + samp);
-            }
-          }
-          mbar_wait(bar(T_L3 + t), ppar);
-          tc_fence_after();
-          uint32_t v[16];
-          tmem_ld16_nowait(tmem_base + (uint32_t)t * HID + lane_off, v);
-          tmem_wait_ld();
-          float dz[4] = {0.f, 0.f, 0.f, 0.f};
-          float loss = 0.f, kl = 0.f, dls[4] = {0.f, 0.f, 0.f, 0.f}, cntv = 0.f;
-          if (samp >= 0) {
-            cntv = 1.f;
-            if (P.mode == MODE_ACTOR_TRAIN) {
-              // agent.py:617-640 with torch.distributions.Normal.log_prob summed over the action dims
-              float lp = 0.f, diff[4], ivar[4];
-              for (int k = 0; k < W.out_dim; ++k) {
-                const float mu = __uint_as_float(v[k]) + sB3[k];
-                const float ls = sLs[k];
-                ivar[k] = __expf(-2.0f * ls);
-                diff[k] = pre_a[k] - mu;
-                lp += -0.5f * diff[k] * diff[k] * ivar[k] - ls - 0.91893853320467f;
-              }
-              const float lpo = pre_lpo;
-              const float ratio = __expf(lp - lpo);
-              const float a = (pre_adv - P.adv_stats[0]) * P.adv_stats[1];
-              const float s1 = ratio * a;
-              const float s2 = fminf(fmaxf(ratio, 1.0f - P.clip), 1.0f + P.clip) * a;
-              loss = -fminf(s1, s2);
-              kl = lpo - lp;
-              const bool inside = ratio >= 1.0f - P.clip && ratio <= 1.0f + P.clip;
-              const float g = (inside || s1 < s2) ? -a * ratio : 0.f;
-              for (int k = 0; k < W.out_dim; ++k) {
-                dz[k] = g * diff[k] * ivar[k];
-                dls[k] = g * (diff[k] * diff[k] * ivar[k] - 1.0f);
-              }
-            } else {
-              // agent.py:643-700, centralised critic: target = mean over agents of identical returns
-              const float vv = __uint_as_float(v[0]) + sB3[0];
-              const float rt = pre_adv;
-              float e = vv - rt;
-              float l = e * e;
-              if (P.use_clipped_value > 0.f) {
-                const float vo = pre_lpo;
-                const float dvc = fminf(fmaxf(vv - vo, -P.clip), P.clip);
-                const float ec = vo + dvc - rt;
-                if (ec * ec > l) { l = ec * ec; e = (fabsf(vv - vo) <= P.clip) ? ec : 0.f; }
-              }
-              loss = 0.5f * l;
-              dz[0] = e;
-            }
-          }
-          // dZ3 tile [128 x 16] bf16, K-major (K = 16): my row's 16 entries = two core-matrix rows
-          const uint4 lo = make_uint4(pack_bf16(dz[0], dz[1]), pack_bf16(dz[2], dz[3]), 0u, 0u);
-          const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-          const size_t off = canon_off(row, 0, kNOut);
-          bf16* z3 = bufZ0 + (size_t)t * kRows * kNOut;
-          *reinterpret_cast<uint4*>(z3 + off) = lo;
-          *reinterpret_cast<uint4*>(z3 + off + 64) = zero;
-          bf16* g3 = P.dZ3t + (size_t)tile * kRows * kNOut;
-          *reinterpret_cast<uint4*>(g3 + off) = lo;
-          *reinterpret_cast<uint4*>(g3 + off + 64) = zero;
-          proxy_fence();
-          tc_fence_before();
-          mbar_arrive(bar(T_Z3 + t));
-          float red[11] = {loss, kl, cntv, dls[0], dls[1], dls[2], dls[3], dz[0], dz[1], dz[2], dz[3]};
-#pragma unroll
-          for (int i = 0; i < 11; ++i) {
-            float x = red[i];
-            for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-            if (lane == 0 && x != 0.f) atomicAdd(&s_red[i], x);
-          }
-          if (tr) tr[5 + t] = clock64();                   // loss(A), loss(B) done
-        }
-      }
-      // ---- dZ2 = dH2 (1 - H2^2), in place over H2: the A operand of the dH1 MMAs
-#pragma unroll 1
-      for (int t = 0; t < nt; ++t) {
-        const long long tile = tile_of(p + t);
-        mbar_wait(bar(T_D2 + t), ppar);
-        tc_fence_after();
-        bf16* sH = bufT0 + (size_t)t * kRows * HID;
-        epi_backward(tmem_base + (uint32_t)t * HID, sH, sH, P.dZ2t + (size_t)tile * kRows * HID, T_Z2 + t);
-        if (tr) tr[7 + t] = clock64();                     // dZ2(A), dZ2(B) done
-      }
-      // ---- dZ1 = dH1 (1 - H1^2): H1 from my own global copy, dZ1 to global only
-#pragma unroll 1
-      for (int t = 0; t < nt; ++t) {
-        const long long tile = tile_of(p + t);
-        mbar_wait(bar(T_D1 + t), ppar);
-        tc_fence_after();
-        epi_backward(tmem_base + (uint32_t)t * HID, P.H1t + (size_t)tile * kRows * HID, nullptr,
-                     P.dZ1t + (size_t)tile * kRows * HID, T_OUT + t);
-        if (tr) tr[9 + t] = clock64();                     // dZ1(A), dZ1(B) done
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (tid < 11 && s_red[tid] != 0.f) atomicAdd(P.stats + tid, (double)s_red[tid]);
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u));
-}
-size_t train2_kernel_smem(int K1p, int stages) {
-  return (size_t)2 * kRows * HID * 2 + (size_t)2 * kRows * K1p * 2 + (size_t)2 * kRows * kNOut * 2 + (size_t)kNOut * HID * 2 +
-         (size_t)stages * kSlabBytes + (size_t)(2 * HID + 2 * kNOut + 16) * 4 + (size_t)T_COUNT * 8 + 16;
-}
-int train2_stages(int K1p) {
-  int st = kMaxStages;
-  while (st > 2 && train2_kernel_smem(K1p, st) > (size_t)227 * 1024) --st;
-  return st;
-}
-
 // dynamic shared memory of mlp_tile_kernel for a net with C input chunks of K1p columns and `stages` ring stages
 size_t tile_kernel_smem(int C, int K1p, int stages) {
   return (size_t)2 * kRows * HID * 2 + (size_t)(C > 1 ? 2 : 1) * kRows * K1p * 2 + (size_t)kRows * kNOut * 2 + (size_t)kNOut * HID * 2 +
@@ -2199,7 +1393,6 @@ struct PackArgs {
   const float* param;
   bf16 *w1_slabs, *w2f_slabs, *w2b_slabs, *w3f, *w3b_slab;
   float *b1, *b2, *b3, *logstd;
-  bf16 *w1c, *w2c, *w3c;     // cluster halves (C == 1 nets), may be null
   AdamArgs adam;             // adam.step != nullptr: thread 0 advances the optimiser's step count (bd_ppo_adam_step)
 };
 __global__ void pack_kernel(const __grid_constant__ PackArgs P) {
@@ -2215,7 +1408,6 @@ __global__ void pack_kernel(const __grid_constant__ PackArgs P) {
     const int col = ks * 16 + kk;
     const float v = col < s.D ? P.param[s.off_w1() + (long long)n * s.din() + c * s.D + col] : 0.f;
     P.w1_slabs[slab * 4096 + canon_off(n, kk, 16)] = __float2bfloat16(v);
-    if (P.w1c != nullptr) P.w1c[(size_t)(n >> 7) * 128 * s.K1p + canon_off(n & 127, col, s.K1p)] = __float2bfloat16(v);
     return;
   }
   long long k = i - n_w1;
@@ -2223,8 +1415,6 @@ __global__ void pack_kernel(const __grid_constant__ PackArgs P) {
     const int slab = (int)(k / 4096), e = (int)(k % 4096), n = e / 16, kk = e % 16;
     const int ks = 4 * (slab & 3) + (slab >> 2);
     P.w2f_slabs[(size_t)slab * 4096 + canon_off(n, kk, 16)] = __float2bfloat16(P.param[s.off_w2() + (long long)n * HID + ks * 16 + kk]);
-    if (P.w2c != nullptr)
-      P.w2c[(size_t)(n >> 7) * 128 * HID + canon_off(n & 127, ks * 16 + kk, HID)] = __float2bfloat16(P.param[s.off_w2() + (long long)n * HID + ks * 16 + kk]);
     // backward slab, same issue order over j: element (i = n, jj = kk) = W2[ks*16 + kk][n]
     P.w2b_slabs[(size_t)slab * 4096 + canon_off(n, kk, 16)] = __float2bfloat16(P.param[s.off_w2() + (long long)(ks * 16 + kk) * HID + n]);
     return;
@@ -2235,7 +1425,6 @@ __global__ void pack_kernel(const __grid_constant__ PackArgs P) {
     const float v = o < s.out_dim ? P.param[s.off_w3() + (long long)o * HID + j] : 0.f;
     P.w3f[canon_off(o, j, HID)] = __float2bfloat16(v);
     P.w3b_slab[canon_off(j, o, 16)] = __float2bfloat16(v);
-    if (P.w3c != nullptr) P.w3c[(size_t)(o >> 3) * 8 * HID + canon_off(o & 7, j, HID)] = __float2bfloat16(v);
     return;
   }
   k -= n_w3;
@@ -2259,7 +1448,6 @@ struct bd_ppo_net {
   long long max_rows, max_tiles;
   // packed weights
   bf16 *w1_slabs = nullptr, *w2f_slabs = nullptr, *w2b_slabs = nullptr, *w3f = nullptr, *w3b_slab = nullptr;
-  bf16 *w1c = nullptr, *w2c = nullptr, *w3c = nullptr;   // cluster halves (C == 1)
   float *b1 = nullptr, *b2 = nullptr, *b3 = nullptr, *logstd = nullptr;
   // tile scratch
   bf16 *Xt = nullptr, *H1t = nullptr, *H2t = nullptr, *dZ2t = nullptr, *dZ1t = nullptr, *dZ3t = nullptr;
@@ -2270,15 +1458,12 @@ struct bd_ppo_net {
   int n1_jobs = 1;               // input chunks are spread over this many role-1 jobs (TMEM: 512 columns)
   double* stats = nullptr;       // [kStatSlots]
   long long* trace = nullptr;    // diagnostics (bd_ppo_set_trace)
-  int fwd_mode = 0;              // bd_ppo_set_forward_mode: 0 = streamed two-tile kernel, 1 = CTA-pair kernel (actor nets)
-  int train_mode = 0;            // bd_ppo_set_train_mode: 0 = one tile in flight (mlp_tile_kernel), 1 = two (mlp_train2_kernel)
   int64_t launches = 0;
 };
 
 namespace {
 void free_net(bd_ppo_net* n) {
   cudaFree(n->w1_slabs); cudaFree(n->w2f_slabs); cudaFree(n->w2b_slabs); cudaFree(n->w3f); cudaFree(n->w3b_slab);
-  cudaFree(n->w1c); cudaFree(n->w2c); cudaFree(n->w3c);
   cudaFree(n->b1); cudaFree(n->b2); cudaFree(n->b3); cudaFree(n->logstd);
   cudaFree(n->Xt); cudaFree(n->H1t); cudaFree(n->H2t); cudaFree(n->dZ2t); cudaFree(n->dZ1t); cudaFree(n->dZ3t);
   cudaFree(n->pw1); cudaFree(n->pw2); cudaFree(n->pw3); cudaFree(n->pb1); cudaFree(n->pb2); cudaFree(n->stats);
@@ -2287,7 +1472,6 @@ NetDev net_dev(const bd_ppo_net* n) {
   NetDev d;
   d.w1_slabs = n->w1_slabs; d.w2f_slabs = n->w2f_slabs; d.w2b_slabs = n->w2b_slabs; d.w3f = n->w3f; d.w3b_slab = n->w3b_slab;
   d.b1 = n->b1; d.b2 = n->b2; d.b3 = n->b3; d.logstd = n->s.has_logstd ? n->logstd : nullptr;
-  d.w1c = n->w1c; d.w2c = n->w2c; d.w3c = n->w3c;
   d.C = n->s.C; d.D = n->s.D; d.K1p = n->s.K1p; d.out_dim = n->s.out_dim;
   return d;
 }
@@ -2334,9 +1518,6 @@ int bd_ppo_net_create(int in_dim, int chunks, int out_dim, int has_logstd, int64
   alloc((void**)&n->w1_slabs, (size_t)chunks * k1s * kSlabBytes);
   alloc((void**)&n->w2f_slabs, 16 * (size_t)kSlabBytes); alloc((void**)&n->w2b_slabs, 16 * (size_t)kSlabBytes);
   alloc((void**)&n->w3f, (size_t)kNOut * HID * 2); alloc((void**)&n->w3b_slab, kSlabBytes);
-  if (chunks == 1) {
-    alloc((void**)&n->w1c, (size_t)HID * n->s.K1p * 2); alloc((void**)&n->w2c, (size_t)HID * HID * 2); alloc((void**)&n->w3c, (size_t)kNOut * HID * 2);
-  }
   alloc((void**)&n->b1, HID * 4); alloc((void**)&n->b2, HID * 4); alloc((void**)&n->b3, kNOut * 4); alloc((void**)&n->logstd, kNOut * 4);
   const size_t T = (size_t)n->max_tiles;
   alloc((void**)&n->Xt, T * chunks * kRows * n->s.K1p * 2);
@@ -2350,8 +1531,6 @@ int bd_ppo_net_create(int in_dim, int chunks, int out_dim, int has_logstd, int64
   alloc((void**)&n->stats, kStatSlots * sizeof(double));
   if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBudget);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kF2SmemBudget);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_train2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_fwd2c_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kDwStages * kDwStageBytes);
   if (prev >= 0 && prev != device) cudaSetDevice(prev);
   if (e != cudaSuccess) {
@@ -2375,16 +1554,6 @@ int bd_ppo_set_trace(bd_ppo_net* n, long long* trace_dev) {
   n->trace = trace_dev;
   return BD_OK;
 }
-int bd_ppo_set_forward_mode(bd_ppo_net* n, int mode) {
-  if (!n || mode < 0 || mode > 1) return pfail(BD_EINVAL, "bd_ppo_set_forward_mode: mode must be 0 or 1");
-  n->fwd_mode = mode;
-  return BD_OK;
-}
-int bd_ppo_set_train_mode(bd_ppo_net* n, int mode) {
-  if (!n || mode < 0 || mode > 1) return pfail(BD_EINVAL, "bd_ppo_set_train_mode: mode must be 0 or 1");
-  n->train_mode = mode;
-  return BD_OK;
-}
 int64_t bd_ppo_net_param_count(const bd_ppo_net* n) { return n ? n->s.count() : 0; }
 int64_t bd_ppo_launch_count(const bd_ppo_net* n) { return n ? n->launches : 0; }
 double* bd_ppo_net_stats(bd_ppo_net* n) { return n ? n->stats : nullptr; }
@@ -2398,7 +1567,6 @@ static int pack_impl(bd_ppo_net* n, const float* flat_params_dev, void* stream, 
   a.s = n->s; a.param = flat_params_dev;
   a.w1_slabs = n->w1_slabs; a.w2f_slabs = n->w2f_slabs; a.w2b_slabs = n->w2b_slabs; a.w3f = n->w3f; a.w3b_slab = n->w3b_slab;
   a.b1 = n->b1; a.b2 = n->b2; a.b3 = n->b3; a.logstd = n->logstd;
-  a.w1c = n->w1c; a.w2c = n->w2c; a.w3c = n->w3c;
   const long long t = pack_threads(n->s);
   pack_kernel<<<(unsigned)((t + 255) / 256), 256, 0, (cudaStream_t)stream>>>(a);
   n->launches++;
@@ -2409,33 +1577,9 @@ static int pack_impl(bd_ppo_net* n, const float* flat_params_dev, void* stream, 
 int bd_ppo_net_pack(bd_ppo_net* n, const float* flat_params_dev, void* stream) { return pack_impl(n, flat_params_dev, stream, nullptr); }
 
 namespace {
-// forward-only launches: the two-tiles-in-flight kernel (BD_PPO_FWD=1tile: the training kernel's forward mode, for A/B runs)
-bool fwd_single_tile() {
-  static const int v = [] { const char* e = getenv("BD_PPO_FWD"); return (e && strcmp(e, "1tile") == 0) ? 1 : 0; }();
-  return v != 0;
-}
-// 0: cluster-pair kernel with resident weights (actor nets with K1p <= 80; bd_ppo_set_forward_mode(n, 1) or
-// BD_PPO_FWD=pair), 1: streamed-weight two-tile kernel (default)
-int fwd_variant(const bd_ppo_net* n) {
-  static const int env_pair = [] { const char* e = getenv("BD_PPO_FWD"); return (e && strcmp(e, "pair") == 0) ? 1 : 0; }();
-  const bool want = env_pair || n->fwd_mode == 1;
-  return (want && n->s.C == 1 && n->w1c != nullptr && fwd2c_kernel_smem(n->s.K1p) <= (size_t)227 * 1024) ? 0 : 1;
-}
+// forward-only launches: mlp_fwd2_kernel, two tiles in flight per CTA
 int launch_fwd2(bd_ppo_net* n, Fwd2Args& a, void* stream, const char* who) {
   a.net = net_dev(n);
-  if (fwd_variant(n) == 0) {
-    const long long ctiles = (a.rows + 2 * kRows - 1) / (2 * kRows);
-    long long clusters = n->sm_count / 2;
-    if (ctiles < 2 * clusters) clusters = (ctiles + 1) / 2;
-    if (clusters < 1) clusters = 1;
-    a.stages = 0;
-    a.trace = n->trace;
-    mlp_fwd2c_kernel<<<(unsigned)(2 * clusters), kThreads, fwd2c_kernel_smem(n->s.K1p), (cudaStream_t)stream>>>(a);
-    n->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return pfail(BD_ECUDA, "%s (pair kernel): %s", who, cudaGetErrorString(e));
-    return BD_OK;
-  }
   const long long tiles = (a.rows + kRows - 1) / kRows;
   // one CTA per SM, every CTA an even number of tiles where possible (a CTA works on pairs)
   long long grid = tiles < n->sm_count ? tiles : n->sm_count;
@@ -2457,31 +1601,14 @@ int bd_ppo_forward(bd_ppo_net* n, const float* obs_dev, int n_envs, int n_agents
                    const float* nmean_dev, const float* nrstd_dev, float nclip, float* out_dev, void* stream) {
   if (!n || !obs_dev || !out_dev) return pfail(BD_EINVAL, "bd_ppo_forward: null argument");
   if (rows <= 0) return BD_OK;
-  if (!fwd_single_tile()) {
-    Fwd2Args f;
-    memset(&f, 0, sizeof(f));
-    f.sample = 0;
-    f.obs = obs_dev; f.N = n_envs; f.M = n_agents; f.idx = (const long long*)idx_dev; f.rows = rows;
-    f.rows_per_sample = n->s.C > 1 ? 1 : n_agents;
-    f.nmean = nmean_dev; f.nrstd = nrstd_dev; f.nclip = nclip;
-    f.out = out_dev;
-    return launch_fwd2(n, f, stream, "bd_ppo_forward");
-  }
-  TileArgs a;
-  memset(&a, 0, sizeof(a));
-  a.net = net_dev(n);
-  a.mode = MODE_FORWARD;
-  a.obs = obs_dev; a.N = n_envs; a.M = n_agents; a.idx = (const long long*)idx_dev; a.rows = rows;
-  a.nmean = nmean_dev; a.nrstd = nrstd_dev; a.nclip = nclip;
-  a.out = out_dev; a.stats = n->stats;
-  const long long tiles = (rows + kRows - 1) / kRows;
-  const int grid = (int)(tiles < n->sm_count ? tiles : n->sm_count);
-  a.stages = tile_stages(n->s.C, n->s.K1p);
-  mlp_tile_kernel<<<grid, kThreads, tile_kernel_smem(n->s.C, n->s.K1p, a.stages), (cudaStream_t)stream>>>(a);
-  n->launches++;
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return pfail(BD_ECUDA, "bd_ppo_forward: %s", cudaGetErrorString(e));
-  return BD_OK;
+  Fwd2Args f;
+  memset(&f, 0, sizeof(f));
+  f.sample = 0;
+  f.obs = obs_dev; f.N = n_envs; f.M = n_agents; f.idx = (const long long*)idx_dev; f.rows = rows;
+  f.rows_per_sample = n->s.C > 1 ? 1 : n_agents;
+  f.nmean = nmean_dev; f.nrstd = nrstd_dev; f.nclip = nclip;
+  f.out = out_dev;
+  return launch_fwd2(n, f, stream, "bd_ppo_forward");
 }
 
 /* Rollout-time policy step of an actor net (`MAPPOActorCritic.step`, agent.py:389-415), one launch: mean = MLP(row),
@@ -2535,19 +1662,9 @@ int bd_ppo_grad(bd_ppo_net* n, int critic, const float* obs_dev, int n_envs, int
   a.stats = n->stats;
   const long long tiles = (rows + kRows - 1) / kRows;
   const int grid = (int)(tiles < n->sm_count ? tiles : n->sm_count);
-  // BD_PPO_TRAIN=2tile (or bd_ppo_set_train_mode(n, 1)): the two-tiles-in-flight kernel.  It reproduces the one-tile
-  // kernel's results and its time (profiles/r2_ppo_train2_trace.txt), so the simpler kernel stays the default.
-  static const bool env_two = [] { const char* e = getenv("BD_PPO_TRAIN"); return e && strcmp(e, "2tile") == 0; }();
-  if ((env_two || n->train_mode == 1) && train2_stages(n->s.K1p) >= 3) {
-    a.stages = train2_stages(n->s.K1p);
-    a.trace = n->trace;
-    const int grid2 = (int)(tiles < 2LL * n->sm_count ? (tiles + 1) / 2 : n->sm_count);
-    mlp_train2_kernel<<<grid2 < 1 ? 1 : grid2, kThreads, train2_kernel_smem(n->s.K1p, a.stages), st>>>(a);
-  } else {
-    a.stages = tile_stages(n->s.C, n->s.K1p);
-    a.trace = n->trace;
-    mlp_tile_kernel<<<grid, kThreads, tile_kernel_smem(n->s.C, n->s.K1p, a.stages), st>>>(a);
-  }
+  a.stages = tile_stages(n->s.C, n->s.K1p);
+  a.trace = n->trace;
+  mlp_tile_kernel<<<grid, kThreads, tile_kernel_smem(n->s.C, n->s.K1p, a.stages), st>>>(a);
   e = cudaGetLastError();
   if (e != cudaSuccess) return pfail(BD_ECUDA, "bd_ppo_grad (tile kernel): %s", cudaGetErrorString(e));
   // ---- weight gradients

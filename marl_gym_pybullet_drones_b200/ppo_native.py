@@ -106,15 +106,6 @@ class PpoNet:
             self._h, _p(param), _p(exp_avg), _p(exp_avg_sq), _p(grad), _p(step), float(lr), float(betas[0]), float(betas[1]),
             float(eps), _p(kl_sum), _p(kl_rows), float(target_kl), _p(gate_count), self._stream()), "bd_ppo_adam_step")
 
-    def set_forward_mode(self, pair: bool):
-        """`forward` / `sample` of an actor net on the CTA-pair kernel (cta_group::2, resident half-weights) or the default
-        streamed two-tile kernel; same results."""
-        self._check(self._lib.bd_ppo_set_forward_mode(self._h, int(bool(pair))), "bd_ppo_set_forward_mode")
-
-    def set_train_mode(self, two_tiles: bool):
-        """`grad` on the two-tiles-in-flight kernel (same results, same speed; kept for comparison) or the default one."""
-        self._check(self._lib.bd_ppo_set_train_mode(self._h, int(bool(two_tiles))), "bd_ppo_set_train_mode")
-
     @property
     def launch_count(self):
         return int(self._lib.bd_ppo_launch_count(self._h))

@@ -39,7 +39,6 @@ from marl_gym_pybullet_drones_b200.ppo_native import PpoNet  # noqa: E402
 net = PpoNet(72, 1, 4, True, 128)
 net.pack(torch.cat([logstd] + [p.detach().reshape(-1) for p in mlp.parameters()]).contiguous())
 obs3 = obs.view(rows // 4, 4, 72)
-net.set_forward_mode("--pair" in sys.argv)
 t2 = timeit(lambda: net.sample(obs3, act, lp, seed=1, offset=2))
 print(f"two-tile tcgen05 sample: {t2:8.1f} us  {flops / t2 / 1e6:7.1f} TFLOP/s (useful flops)  [bd_ppo_sample]")
 out = torch.empty(rows, 4, device="cuda")

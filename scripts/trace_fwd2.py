@@ -19,7 +19,6 @@ mlp = MLP(72, 4, [256, 256], "tanh").cuda()
 logstd = torch.full((4,), -0.5, device="cuda")
 obs = torch.randn(rows // 4, 4, 72, device="cuda")
 net = PpoNet(72, 1, 4, True, 128)
-net.set_forward_mode("--pair" in sys.argv)
 net.pack(torch.cat([logstd] + [p.detach().reshape(-1) for p in mlp.parameters()]).contiguous())
 act = torch.empty(rows, 4, device="cuda")
 lp = torch.empty(rows, device="cuda")
@@ -34,9 +33,7 @@ net._lib.bd_ppo_set_trace(net._h, None)
 t = trace.cpu().numpy()
 pairs = [j for j in range(32) if t[j, 0] != 0]
 t0 = t[pairs[0], 0]
-pairk = "--pair" in sys.argv
-E = ["start", "L1A ready", "H1A done", "L1B ready", "H1B done", "L2A ready", "H2A done", "L2B ready", "H2B done", "L3A ready",
-     "XA' staged", "outA done", "L3B ready", "XB' staged", "outB done"] if pairk else ["start", "L1A done", "H1A done", "XA' staged", "L1B done", "H1B done", "XB' staged", "L2A done", "H2A done", "-",
+E = ["start", "L1A done", "H1A done", "XA' staged", "L1B done", "H1B done", "XB' staged", "L2A done", "H2A done", "-",
      "L2B done", "H2B done", "-", "L3A done", "outA done", "L3B done", "outB done"]
 Mn = ["start", "OUT A ok", "OUT B ok", "L1A issued", "L1B issued", "H1A ready", "H1B ready", "L2A issued", "L2B issued", "H2A ready",
       "H2B ready", "L3A issued", "L3B issued"]

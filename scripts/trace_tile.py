@@ -28,7 +28,6 @@ else:
     net = PpoNet(D, 1, A, True, samples * M)
     net.pack(t._flat([torch.full((A,), -0.5, device="cuda")] + list(t._mlp(D, A, 6).parameters())))
 gr = torch.zeros(net.param_count, device="cuda")
-net.set_train_mode("--two" in sys.argv)
 
 
 def one():
@@ -48,13 +47,11 @@ one()
 torch.cuda.synchronize()
 net._lib.bd_ppo_set_trace(net._h, None)
 tr = trace.cpu().numpy()
-two = "--two" in sys.argv
-names = ["pair start", "H1(A) done", "H1(B) done", "H2(A) done", "H2(B) done", "loss(A) done", "loss(B) done", "dZ2(A) done",
-         "dZ2(B) done", "dZ1(A) done", "dZ1(B) done"] if two else ["tile start", "inputs staged", "L1 complete", "H1 written", "L2 complete", "H2 written", "L3 complete", "loss done",
+names = ["tile start", "inputs staged", "L1 complete", "H1 written", "L2 complete", "H2 written", "L3 complete", "loss done",
          "dH2 complete", "dZ2 written", "dH1 complete", "dZ1 written", "(loss inputs in)", "(dZ3 handed over)"]
 rows = [j for j in range(16) if tr[j, 0] != 0]
 for j in rows[:3] + rows[-1:]:
-    print(f"{'pair' if two else 'tile'} {j} of CTA 0 (cycles since it started, delta)")
+    print(f"tile {j} of CTA 0 (cycles since it started, delta)")
     prev = tr[j, 0]
     for k, nme in sorted(enumerate(names), key=lambda kn: tr[j, kn[0]]):
         if tr[j, k]:
@@ -62,4 +59,4 @@ for j in rows[:3] + rows[-1:]:
             prev = tr[j, k]
 if len(rows) > 2:
     per = (tr[rows[-1], 0] - tr[rows[1], 0]) / (len(rows) - 2)
-    print("cycles per tile (steady):", per / 2 if two else per)
+    print("cycles per tile (steady):", per)

@@ -79,10 +79,9 @@ def test_gae_kernel_matches_reference_scan(T, N):
         assert abs(float(st[1]) - 1.0 / (want_adv.std() + 1e-8)) <= 1e-4 / (want_adv.std() + 1e-8)   # np.std: ddof = 0
 
 
-@pytest.mark.parametrize("pair", [False, True])
 @pytest.mark.parametrize("M,D,A,samples,critic", [(4, 72, 4, 300, False), (2, 72, 4, 1000, False), (4, 72, 4, 517, True),
                                                   (2, 27, 1, 260, False), (1, 72, 4, 129, True), (16, 72, 4, 200, True)])
-def test_forward_matches_torch(M, D, A, samples, critic, pair):
+def test_forward_matches_torch(M, D, A, samples, critic):
     from marl_gym_pybullet_drones_b200.ppo_native import PpoNet
     T, N = 6, 64
     obs, act, g = _rollout(T, N, M, D, A, 1)
@@ -98,7 +97,6 @@ def test_forward_matches_torch(M, D, A, samples, critic, pair):
         rows = samples * M
         x = obs[:T].reshape(T * N, M, D)[idx].reshape(rows, D)
     params = ([torch.full((A,), -0.5, device="cuda")] if not critic else []) + list(mlp.parameters())
-    net.set_forward_mode(pair)          # actor nets: the CTA-pair kernel (cta_group::2); critic nets ignore it
     net.pack(_flat(params))
     out = net.forward(obs, N, M, rows, idx=idx)
     want = mlp(x)
@@ -114,8 +112,7 @@ def test_forward_matches_torch(M, D, A, samples, critic, pair):
     net.close()
 
 
-@pytest.mark.parametrize("pair", [False, True])
-def test_forward_many_tiles_per_cta(pair):
+def test_forward_many_tiles_per_cta():
     """More tiles than 2 x SMs, odd count, ragged last tile: every CTA of the two-tiles-in-flight kernel runs several
     pairs plus a single; actor rows and critic rows (M input chunks)."""
     from marl_gym_pybullet_drones_b200.ppo_native import PpoNet
@@ -125,7 +122,6 @@ def test_forward_many_tiles_per_cta(pair):
     idx = torch.randint(0, T * N, (samples,), device="cuda", generator=g)
     mlp = _mlp(D, A, 4)
     net = PpoNet(D, 1, A, True, samples * M)
-    net.set_forward_mode(pair)
     net.pack(_flat([torch.full((A,), -0.5, device="cuda")] + list(mlp.parameters())))
     out = net.forward(obs, N, M, samples * M, idx=idx)
     with torch.no_grad():
@@ -142,9 +138,8 @@ def test_forward_many_tiles_per_cta(pair):
     cnet.close()
 
 
-@pytest.mark.parametrize("pair", [False, True])
 @pytest.mark.parametrize("N,M,D,A", [(700, 4, 72, 4), (50, 2, 27, 1), (40000, 4, 72, 4), (3, 16, 72, 4)])
-def test_sample_matches_torch(N, M, D, A, pair):
+def test_sample_matches_torch(N, M, D, A):
     """`MAPPOActorCritic.step` (agent.py:389-415): act = mean + exp(logstd) eps, logp = summed Normal log-density;
     mean within the forward tolerance, act / logp exact given the mean and the noise (fp32, <= 1e-5)."""
     from marl_gym_pybullet_drones_b200.ppo_native import PpoNet
@@ -153,7 +148,6 @@ def test_sample_matches_torch(N, M, D, A, pair):
     mlp = _mlp(D, A, 8)
     logstd = torch.linspace(-0.7, -0.2, A, device="cuda")
     net = PpoNet(D, 1, A, True, 128)
-    net.set_forward_mode(pair)
     net.pack(_flat([logstd] + list(mlp.parameters())))
     noise = torch.randn((N, M, A), device="cuda", generator=g)
     act, logp, mean = (torch.empty((N, M, A), device="cuda"), torch.empty((N, M, 1), device="cuda"),
@@ -205,9 +199,8 @@ def _actor_reference(mlp, logstd, obs, act, logp_old, adv_n, idx, T, N, M, D, A,
     return policy_loss, entropy_loss, kl
 
 
-@pytest.mark.parametrize("two_tiles", [False, True])
 @pytest.mark.parametrize("M,samples", [(4, 1024), (2, 333), (1, 128), (4, 128 * 148 * 3 // 4 + 5)])
-def test_actor_gradient_matches_autograd(M, samples, two_tiles):
+def test_actor_gradient_matches_autograd(M, samples):
     from marl_gym_pybullet_drones_b200 import ppo_native
     from marl_gym_pybullet_drones_b200.ppo_native import PpoNet
     T, N, D, A = 8, (200 if samples <= 1600 else 2000), 72, 4
@@ -231,7 +224,6 @@ def test_actor_gradient_matches_autograd(M, samples, two_tiles):
     params = [logstd] + list(mlp.parameters())
     want = torch.autograd.grad(pl + ent * el, params)
     net = PpoNet(D, 1, A, True, samples * M)
-    net.set_train_mode(two_tiles)       # both forward / loss / backward kernels: one tile in flight (default), two tiles
     net.pack(_flat(params))
     grad = torch.zeros(net.param_count, device="cuda")
     net.grad(grad, obs, N, M, idx, samples, critic=False, act=act, logp_old=logp_old, adv=adv, adv_stats=stats2, clip=clip,
@@ -252,9 +244,8 @@ def test_actor_gradient_matches_autograd(M, samples, two_tiles):
     net.close()
 
 
-@pytest.mark.parametrize("two_tiles", [False, True])
 @pytest.mark.parametrize("M,samples,clipped", [(4, 700, False), (2, 256, True), (16, 150, False), (1, 130, False)])
-def test_critic_gradient_matches_autograd(M, samples, clipped, two_tiles):
+def test_critic_gradient_matches_autograd(M, samples, clipped):
     from marl_gym_pybullet_drones_b200.ppo_native import PpoNet
     T, N, D = 8, 100, 72
     obs, _, g = _rollout(T, N, M, D, 4, 9)
@@ -274,7 +265,6 @@ def test_critic_gradient_matches_autograd(M, samples, clipped, two_tiles):
     params = list(mlp.parameters())
     want = torch.autograd.grad(loss, params)
     net = PpoNet(D, M, 1, False, samples)
-    net.set_train_mode(two_tiles)
     net.pack(_flat(params))
     grad = torch.zeros(net.param_count, device="cuda")
     net.grad(grad, obs, N, M, idx, samples, critic=True, ret=ret, v_old=v_old, clip=0.2, use_clipped_value=clipped)
